@@ -240,6 +240,16 @@ def sweep256(dev, model, batches, n_steps, seed):
     return rows
 
 
+def dump_step_outputs(out_dir, loss):
+    """What a training step returns to its caller, as float32 .npy files for output-for-output comparisons of two builds:
+    loss.npy.  The weights the step leaves are not dumped: the weight gradients are summed with float atomics, and Adam at
+    lr 0.02 amplifies that ordering noise until, after the ~90 steps of a default run, two runs of the same build hold
+    weights half their norm apart (measured on a B200 at a 1000 W power limit), while their losses agree to ~0.5%."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().cpu().numpy())
+
+
 def conv_only_oplist(plan):
     """Every convolution / weight-gradient launch of one training step as a stand-alone op list (the fused conv+BN ops
     contribute their convolution only: d3fk_convbn_params starts with the d3fk_conv_params)."""
@@ -330,6 +340,8 @@ def run_d3fk(args):
         ms = t.item()
     value = world * B * args.steps / (ms / 1e3)
     final_loss = float(loss)
+    if args.dump_outputs and rank == 0:        # before the e2e leg below trains the model further
+        dump_step_outputs(args.dump_outputs, loss)
 
     # ---------------- end to end through the public API with host buffers ("e2e")
     # Every step copies its input batch from pinned host memory and reads its loss back to the host.  As a training
@@ -563,7 +575,12 @@ def main():
                     help="which measurement becomes the headline metric/value of the JSON line (train = BASELINE configs[1])")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--main-priority", type=int, default=int(os.environ.get("D3FK_MAIN_PRIORITY", "0")))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed training step returned to DIR/<name>.npy "
+                         "(float32): loss.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "d3fk":
+        ap.error("--dump-outputs dumps the d3fk training step (--impl d3fk)")
     if args.impl == "reference":
         run_reference(args)
     else:
