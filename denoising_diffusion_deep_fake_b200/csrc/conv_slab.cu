@@ -460,7 +460,9 @@ static int launch_conv_slab_bn(const Gather& g, const d3fk_conv_params* p, cudaS
   if (occ * tmem_cols > 512) occ = 512 / tmem_cols;
   if (occ < 1) occ = 1;
   int grid = ss.total < g_num_sms * occ ? ss.total : g_num_sms * occ;
-  if (g_verbose) fprintf(stderr, "[d3fk] slab<%d> mode=%d M=%d C=%d Cout=%d W=%d S=%d stages=%d smem=%d grid=%d total=%d flat=%d RT=%d\n", BN, g.mode, g.M, C, p->Cout, ss.W, ss.S, ss.stages, smem, grid, ss.total, ss.flat, ss.RT);
+  // epi: as the conv_tc line (0 plain, 2 BN-backward sums, 3 affine / bias: the AFF variant); the slab kernel has no fused BN
+  const int epi = p->bw_x ? 2 : AFF ? 3 : 0;
+  if (g_verbose) fprintf(stderr, "[d3fk] slab<%d> mode=%d M=%d C=%d Cout=%d W=%d S=%d stages=%d smem=%d grid=%d total=%d flat=%d RT=%d epi=%d\n", BN, g.mode, g.M, C, p->Cout, ss.W, ss.S, ss.stages, smem, grid, ss.total, ss.flat, ss.RT, epi);
   launch_k(conv_slab_kernel<BN, KSTEPS, AFF>, dim3(grid), dim3(SlabCfg<BN>::THREADS), (size_t)smem, s, dim3(1, 1, 1), tmA, tmB, e, ss,
            make_fastdiv((uint32_t)g.Wo), make_fastdiv((uint32_t)g.Ho), g_dev_error_flag);
   count_launch();

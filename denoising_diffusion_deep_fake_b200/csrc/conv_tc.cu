@@ -675,7 +675,9 @@ static int launch_conv_tc_bn(const Gather& g, const d3fk_conv_params* p, cudaStr
     grid = ts.total;
     t_fuse->taken = true;
   }
-  if (g_verbose) fprintf(stderr, "[d3fk] conv<%d,%d> mode=%d M=%d K=%d Cout=%d tiles=%d KS=%d kbps=%d grid=%d fuse=%d\n", BN, PATH, g.mode, g.M, g.K, p->Cout, tiles, ts.KS, ts.kb_per_split, grid, (int)fuse);
+  // epi = the FUSE template argument of the kernel launched below: 0 plain, 1 fused BN, 2 BN-backward sums, 3 eval affine / bias
+  const int epi = p->bw_x ? 2 : fuse ? 1 : (p->scale || p->shift) ? 3 : 0;
+  if (g_verbose) fprintf(stderr, "[d3fk] conv<%d,%d> mode=%d M=%d K=%d Cout=%d tiles=%d KS=%d kbps=%d grid=%d fuse=%d epi=%d\n", BN, PATH, g.mode, g.M, g.K, p->Cout, tiles, ts.KS, ts.kb_per_split, grid, (int)fuse, epi);
   cudaError_t le;
   if (p->bw_x)
     le = launch_k(conv_tc_kernel<BN, PATH, 2>, dim3(grid), dim3(TC_THREADS), ConvCfg<BN, PATH, 2>::SMEM, s, dim3(ts.KS, 1, 1), g,
