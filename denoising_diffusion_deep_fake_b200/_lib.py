@@ -58,7 +58,7 @@ class PackParams(C.Structure):
 class BnParams(C.Structure):
     _fields_ = [("dtype", i32), ("C", i32), ("relu", i32), ("mask_from_x", i32), ("count", i64),
                 ("x", vp), ("y", vp), ("res", vp),
-                ("ldx", i32), ("ldy", i32), ("ldr", i32), ("_pad1", i32),
+                ("ldx", i32), ("ldy", i32), ("ldr", i32), ("frozen", i32),
                 ("stats", vp), ("gamma", vp), ("beta", vp),
                 ("running_mean", vp), ("running_var", vp), ("num_batches_tracked", vp),
                 ("eps", f32), ("momentum", f32),

@@ -755,6 +755,7 @@ static int launch_conv_windowed(const d3fk_conv_params* p, cudaStream_t s) {
 
 int try_launch_conv_slab(const Gather& g, const d3fk_conv_params* p, cudaStream_t s);   // conv_slab.cu
 int try_launch_head_conv(const d3fk_conv_params* p, cudaStream_t s);
+int try_launch_stem_dgrad(const d3fk_conv_params* p, cudaStream_t s);   // stem_dgrad.cu
 int launch_conv_tc(const d3fk_conv_params* p, cudaStream_t s) {
   Gather g;
   int rc = make_gather(g, p->src0, p->src1, p->c0, p->c1, p->ld0, p->ld1, p->up0, p->B, p->Hi, p->Wi, p->Ho, p->Wo, p->kh,
@@ -767,6 +768,8 @@ int launch_conv_tc(const d3fk_conv_params* p, cudaStream_t s) {
   if (p->mode == 2) return launch_conv_windowed(p, s);
   const int head = try_launch_head_conv(p, s);          // 16 -> 3 channels, fp32 NCHW out: CUDA cores (head_conv.cu)
   if (head) return head < 0 ? head : D3FK_OK;
+  const int stem = try_launch_stem_dgrad(p, s);         // 7x7 / stride-2 input gradient, 64 -> 3 channels, fp32 NCHW out
+  if (stem) return stem < 0 ? stem : D3FK_OK;
   const int slab = try_launch_conv_slab(g, p, s);
   if (slab) return slab < 0 ? slab : D3FK_OK;
   TileSched box;

@@ -127,7 +127,8 @@ __global__ void bn_finalize_kernel(d3fk_bn_params p) {
   if (c == 0 && p.num_batches_tracked) *p.num_batches_tracked += 1;
 }
 
-// eval mode: scale/shift from running statistics (folded into the conv epilogue)
+// eval mode: scale/shift from running statistics (folded into the conv epilogue).  mean / invstd set (frozen-BN plans): the
+// running statistics are published there too, for the backward's xhat = (x - running_mean) * invstd_run.
 __global__ void bn_fold_kernel(d3fk_bn_params p) {
   pdl_enter();
   int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -136,6 +137,8 @@ __global__ void bn_fold_kernel(d3fk_bn_params p) {
   float sc = p.gamma[c] * invstd;
   p.scale[c] = sc;
   p.shift[c] = p.beta[c] - p.running_mean[c] * sc;
+  if (p.mean) p.mean[c] = p.running_mean[c];
+  if (p.invstd) p.invstd[c] = invstd;
 }
 
 // y = relu?(x*scale + shift + res).  With p.stats set (train forward) the batch statistics are finalised here:
@@ -236,7 +239,9 @@ __device__ __forceinline__ void lds_volatile_f4(uint32_t addr, float (&v)[4]) {
 // per-channel sums of dy' and dy'*xhat ; dy' = relu ? (act>0 ? dy : 0) : dy.
 // Lanes of a warp that own the same channel vector are folded with shuffles, warps with one shared-memory
 // slot each, the block with one double atomic per channel.
-template <typename T, typename Acc, bool XMASK>
+// FROZEN (BatchNorm on its running statistics): dx = gamma*invstd*dy' does not depend on the sums, so the same pass also
+// writes dx (and dres = dy') — BN backward in one read of dy, x (and act) and one write.
+template <typename T, typename Acc, bool XMASK, bool FROZEN = false>
 __device__ __forceinline__ void bn_bwd_reduce_body(const d3fk_bn_params& p, double* sred) {
   constexpr int V = Vec<T>::N;
   const int C = p.C, cvs = C / V;
@@ -248,9 +253,12 @@ __device__ __forceinline__ void bn_bwd_reduce_body(const d3fk_bn_params& p, doub
 #pragma unroll
   for (int i = 0; i < V; ++i) { s1[i] = 0; s2[i] = 0; }
   constexpr bool xmask = XMASK;                      // p.relu && p.mask_from_x, resolved at launch (register budget)
-  float* s_ms = reinterpret_cast<float*>(sred);      // [2][C] scale, shift — aliases the reduction slots, dead until the loop ends
-  if (xmask) {
-    for (int ch = threadIdx.x; ch < C; ch += blockDim.x) { s_ms[ch] = p.scale[ch]; s_ms[C + ch] = p.shift[ch]; }
+  float* s_ms = reinterpret_cast<float*>(sred);      // [3][C] scale, shift, gamma*invstd — aliases the reduction slots, dead until the loop ends
+  if (xmask || FROZEN) {
+    for (int ch = threadIdx.x; ch < C; ch += blockDim.x) {
+      if (xmask) { s_ms[ch] = p.scale[ch]; s_ms[C + ch] = p.shift[ch]; }
+      if (FROZEN) s_ms[2 * C + ch] = __ldg(p.gamma + ch) * __ldg(p.invstd + ch);
+    }
     __syncthreads();
   }
   const uint32_t ms_addr = (uint32_t)__cvta_generic_to_shared(s_ms + c);
@@ -297,6 +305,7 @@ __device__ __forceinline__ void bn_bwd_reduce_body(const d3fk_bn_params& p, doub
                 float xh = (xv[i] - mean[i]) * istd[i];
                 s1[i] += (Acc)g;
                 s2[i] += (Acc)(g * xh);
+                gv[i] = g;
               }
             }
           } else {
@@ -309,13 +318,27 @@ __device__ __forceinline__ void bn_bwd_reduce_body(const d3fk_bn_params& p, doub
               float xh = (xv[i] - mean[i]) * istd[i];
               s1[i] += (Acc)g;
               s2[i] += (Acc)(g * xh);
+              gv[i] = g;
             }
+          }
+          if (FROZEN) {
+            const long long pix = pix0 + u * pstride;
+            float o[V];
+#pragma unroll
+            for (int i4 = 0; i4 < V; i4 += 4) {
+              float kA[4];
+              lds_volatile_f4(ms_addr + 8u * (uint32_t)C + 4u * i4, kA);
+#pragma unroll
+              for (int j = 0; j < 4; ++j) o[i4 + j] = fmaf(kA[j], gv[i4 + j], 0.f);   // = bn_bwd_apply's A*g' + (0*(x-mean) + 0)
+            }
+            store_vec<T>((T*)p.dx + pix * p.lddx + c, o);
+            if (p.dres) store_vec<T>((T*)p.dres + pix * p.lddres + c, gv);
           }
         }
       }
     }
   }
-  if (xmask) __syncthreads();     // the staged scale / shift are dead: the slots below overwrite them
+  if (xmask || FROZEN) __syncthreads();     // the staged scale / shift / gamma*invstd are dead: the slots below overwrite them
   // fold lanes that share cv (lane stride cvs) when a warp holds several pixel rows
   if (cvs < 32) {
 #pragma unroll
@@ -361,6 +384,15 @@ __global__ void __launch_bounds__(256, BN_BWD_OCC(T)) bn_bwd_reduce_kernel(d3fk_
   bn_bwd_reduce_body<T, Acc, XMASK>(p, sred_dyn);
 }
 
+// frozen BN backward, one pass: dx (and dres) written, sum(dy') / sum(dy' * xhat) accumulated; bn_bwd_finalize writes dgamma / dbeta
+// (two blocks per SM on the bf16 engine: the dx / dres stores need the registers the three-block budget of the reduce kernel lacks)
+template <typename T, typename Acc, bool XMASK>
+__global__ void __launch_bounds__(256, sizeof(T) == 2 ? 2 : 1) bn_bwd_frozen_kernel(d3fk_bn_params p) {
+  pdl_enter();
+  extern __shared__ double sred_dyn[];  // [warps][2][C]
+  bn_bwd_reduce_body<T, Acc, XMASK, true>(p, sred_dyn);
+}
+
 __global__ void bn_bwd_finalize_kernel(d3fk_bn_params p) {
   pdl_enter();
   int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -369,6 +401,7 @@ __global__ void bn_bwd_finalize_kernel(d3fk_bn_params p) {
   double s1 = p.bstats[c], s2 = p.bstats[p.C + c];
   if (p.dbeta) p.dbeta[c] = (float)s1;
   if (p.dgamma) p.dgamma[c] = (float)s2;
+  if (!p.coef) return;
   p.coef[c] = p.gamma[c] * p.invstd[c];
   p.coef[p.C + c] = (float)(s1 / n);
   p.coef[2 * p.C + c] = (float)(s2 / n);
@@ -401,8 +434,9 @@ __device__ __forceinline__ void bn_bwd_apply_body(const d3fk_bn_params& p, float
     const float is = __ldg(p.invstd + ch);
     const float A = __ldg(p.gamma + ch) * is;
     s_k[ch] = A;
-    s_k[p.C + ch] = -A * is * (float)(s2 / n);
-    s_k[2 * p.C + ch] = -A * (float)(s1 / n);
+    // frozen (running statistics): the normalisation is a constant affine map, dx = A*dy'
+    s_k[p.C + ch] = p.frozen ? 0.f : -A * is * (float)(s2 / n);
+    s_k[2 * p.C + ch] = p.frozen ? 0.f : -A * (float)(s1 / n);
     s_k[3 * p.C + ch] = __ldg(p.mean + ch);
     if (XMASK) {
       s_k[4 * p.C + ch] = p.scale[ch];
@@ -1138,7 +1172,35 @@ int launch_bn_bwd_apply(const d3fk_bn_params* p, cudaStream_t s) {
   count_launch();
   return check_launch("bn_bwd_apply");
 }
+static int launch_bn_bwd_frozen(const d3fk_bn_params* p, cudaStream_t s) {
+  D3FK_CHECK_ARG(p->C % 8 == 0 && p->C <= 1024, "C must be a multiple of 8, <= 1024");
+  D3FK_CHECK_ARG(p->dx && p->bstats && p->gamma && p->invstd && p->mean, "frozen BN backward: dx, bstats, gamma, mean, invstd");
+  const int V = p->dtype == D3FK_F32 ? 4 : 8;
+  const int cvs = p->C / V;
+  D3FK_CHECK_ARG((cvs & (cvs - 1)) == 0 && cvs <= 256, "C/V must be a power of two <= 256");
+  const int threads = 256;
+  const int rows = threads / cvs;
+  int grid = cdiv(p->count, (long long)rows * 8);
+  if (grid > kSMs * 8) grid = kSMs * 8;
+  if (grid < 1) grid = 1;
+  const int slotC = cvs < 32 ? p->C : 32 * V;
+  size_t smem = (size_t)(threads / 32) * 2 * slotC * sizeof(double);
+  if (smem < 3 * (size_t)p->C * sizeof(float)) smem = 3 * (size_t)p->C * sizeof(float);
+  const bool xm = p->relu && p->mask_from_x;
+  D3FK_CHECK_ARG(!xm || (p->scale && p->shift), "mask_from_x needs scale / shift");
+  if (p->dtype == D3FK_F32) {
+    if (xm) launch_k(bn_bwd_frozen_kernel<float, double, true>, dim3(grid), dim3(threads), smem, s, dim3(1, 1, 1), *p);
+    else launch_k(bn_bwd_frozen_kernel<float, double, false>, dim3(grid), dim3(threads), smem, s, dim3(1, 1, 1), *p);
+  } else if (p->dtype == D3FK_BF16) {
+    if (xm) launch_k(bn_bwd_frozen_kernel<__nv_bfloat16, float, true>, dim3(grid), dim3(threads), smem, s, dim3(1, 1, 1), *p);
+    else launch_k(bn_bwd_frozen_kernel<__nv_bfloat16, float, false>, dim3(grid), dim3(threads), smem, s, dim3(1, 1, 1), *p);
+  } else return set_error(D3FK_ERR_ARG, "bad dtype");
+  count_launch();
+  int rc = check_launch("bn_bwd_frozen");
+  return rc ? rc : launch_bn_bwd_finalize(p, s);
+}
 int launch_bn_bwd(const d3fk_bn_params* p, cudaStream_t s) {
+  if (p->frozen) return launch_bn_bwd_frozen(p, s);
   D3FK_CHECK_ARG(p->C % 8 == 0 && p->C <= 1024, "C must be a multiple of 8, <= 1024");
   const int V = p->dtype == D3FK_F32 ? 4 : 8;
   const int cvs = p->C / V;

@@ -1,12 +1,17 @@
 """Op-list plans for the resnet34 U-Net (smp.Unet restated in SURVEY Appendix A).
 
-A plan is built once per (batch, H, W, dtype, train/eval) and owns every intermediate buffer; running
+A plan is built once per (batch, H, W, dtype, variant) and owns every intermediate buffer; running
 it is ONE call into libd3fk (`d3fk_run`) that enqueues the whole forward (or backward) on the
 current CUDA stream — no tracing compiler, no per-layer Python in the hot loop, CUDA-graph safe.
 
 Topology follows torchvision/models/resnet.py:89-105,197-205,266-278 (encoder) and smp's
 UnetDecoder / DecoderBlock / SegmentationHead (SURVEY Appendix A1); the call being replaced is
 `self.model(image_noisy)` at d3f/train_denoiser/lit_module.py:117 and its autograd backward.
+
+Variants: the training plan (batch statistics, backward), the eval plan (BatchNorm folded into the convolutions, forward only)
+and the frozen-BN plan (`frozen=True`: BatchNorm on its running statistics as in eval mode, nothing updates them, with a
+backward — eval-mode autograd).  `want_dx=True` adds the input gradient to a plan's backward: the stem's dgrad, written as fp32
+NCHW into the pointer `run_backward(dx=...)` patches in.
 """
 import os
 
@@ -132,8 +137,10 @@ class T:
 
 
 class UnetPlan:
-    def __init__(self, params, buffers, B, H, W, dtype, device, training, grad_arena=None, grad_offsets=None):
-        """params/buffers: dict name -> tensor (the module's own parameters / BN buffers, fp32)."""
+    def __init__(self, params, buffers, B, H, W, dtype, device, training, grad_arena=None, grad_offsets=None, frozen=False,
+                 want_dx=False):
+        """params/buffers: dict name -> tensor (the module's own parameters / BN buffers, fp32).  frozen (with training=False):
+        the frozen-BN plan.  want_dx (plans with a backward): the backward also produces the gradient of the input image."""
         if H % 32 or W % 32:
             raise RuntimeError(f"Wrong input shape height={H}, width={W}. Expected image height and width "
                                f"divisible by 32.")
@@ -142,6 +149,11 @@ class UnetPlan:
         self.tdtype = torch.float32 if dtype == _lib.F32 else torch.bfloat16
         self.device = torch.device(device)
         self.training = training
+        self.frozen = bool(frozen) and not training
+        self.has_backward = training or self.frozen
+        if want_dx and not self.has_backward:
+            raise ValueError("want_dx needs a plan with a backward (training or frozen)")
+        self.want_dx = bool(want_dx)
         self.params, self.buffers = params, buffers
         self.keep = []          # every tensor the op lists point into
         self.generation = 0
@@ -153,14 +165,14 @@ class UnetPlan:
         self._alloc_bn()
         # fp32 scratch for split-K convolutions (deep layers whose output tiles cannot fill 148 SMs)
         self.ws = self._new((SPLITK_WS_BYTES // 4,), torch.float32) if dtype == _lib.BF16 else None
-        self.grad_arena, self.grad_offsets = (grad_arena, grad_offsets) if training else (None, None)
+        self.grad_arena, self.grad_offsets = (grad_arena, grad_offsets) if self.has_backward else (None, None)
         self.pack_ops = _lib.OpList(self._build_pack())
         self.prepacked_version = None   # Unet._weights_version() the packed operands were last produced for (train.StepOverlap)
         self.saved = {}
         fwd = self._build_forward()
         self.fwd_ops = _lib.OpList(fwd)
         self.bwd_segments = None
-        if training:
+        if self.has_backward:
             self.bwd_segments = [_lib.OpList(seg) for seg in self._build_backward()]
         self._record_param_ptrs()
 
@@ -177,7 +189,9 @@ class UnetPlan:
             cout_pad = DY_PAD if c.cout == 3 else c.cout
             taps = c.k * c.k
             self.w_fwd[c.name] = self._new((c.cout, taps * cin_pad), self.tdtype)
-            if self.training and c is not self.stem:
+            if self.has_backward and (c.name != self.stem.name or self.want_dx):
+                # the stem's dgrad operand [3][7][7][64] only where the input gradient is wanted (compared by name: all_convs()
+                # builds its own ConvSpec objects)
                 self.w_dgrad[c.name] = self._new((c.cin, taps * cout_pad), self.tdtype)
         # bf16 engine: the 7x7 / stride-2 stem runs as a space-to-depth convolution (conv mode 2, include/d3fk.h) whenever
         # its 128-pixel output tile is a (w, h, n) box — K = 256 by TMA instead of K = 392 by per-thread gather (65 -> 25 us)
@@ -297,11 +311,12 @@ class UnetPlan:
                 bucket_ops.append(stem_op)
             self.pack_bucket_ops.append(_lib.OpList(bucket_ops))
         if not self.training:
+            # frozen plans also publish the running statistics as mean / invstd: the backward's xhat rows
+            keys = ("dtype", "C", "eps", "gamma", "beta", "running_mean", "running_var", "scale", "shift") + \
+                (("mean", "invstd") if self.frozen else ())
             for c in self.convs:
                 if c.bn:
-                    ops.append(make_op(_lib.OP_BN_FOLD, **{k: v for k, v in self._bn_common(c).items()
-                                                          if k in ("dtype", "C", "eps", "gamma", "beta", "running_mean",
-                                                                   "running_var", "scale", "shift")}))
+                    ops.append(make_op(_lib.OP_BN_FOLD, **{k: v for k, v in self._bn_common(c).items() if k in keys}))
         return ops
 
     # ------------------------------------------------------------------ forward
@@ -339,7 +354,8 @@ class UnetPlan:
 
     def _conv_bn_act(self, ops, c, src0, src1=None, up0=0, relu=1, res=None, lane=0, override=None):
         """conv -> BN -> (+res) -> ReLU.  Train: raw conv output + batch statistics in the conv epilogue,
-        finalize, one fused apply pass.  Eval: BN folded into the conv epilogue.  Returns the activation.
+        finalize, one fused apply pass.  Eval: BN folded into the conv epilogue.  Frozen: the raw conv output is kept for
+        backward and one apply pass uses the folded scale / shift (no statistics, no barrier).  Returns the activation.
         lane != 0: the op runs on a branch stream of d3fk_run (always in its two-kernel form: a branch never waits on a
         grid-wide barrier)."""
         Hi = src0.H * (2 if up0 else 1)
@@ -348,21 +364,23 @@ class UnetPlan:
         Wo = (Wi + 2 * c.pad - c.k) // c.stride + 1
         act = T(self, self.B, Ho, Wo, c.cout)
         self.keep.append(act.t)
-        if not self.training:
+        if not self.has_backward:
             op, _, _ = self._conv_op(c, src0, src1, up0, out=act, relu=relu, res=res, affine=True, lane=lane, override=override)
             ops.append(op)
             return act
         raw = T(self, self.B, Ho, Wo, c.cout)
         self.keep.append(raw.t)
-        conv_fields = self._conv_fields(c, src0, src1, up0, out=raw, stats=True, override=override)
+        conv_fields = self._conv_fields(c, src0, src1, up0, out=raw, stats=not self.frozen, override=override)
         bn = self._bn_common(c)
         bn.update(count=raw.count, relu=relu, x=raw.ptr, ldx=raw.ld, y=act.ptr, ldy=act.ld)
+        if self.frozen:
+            bn.update(stats=None, frozen=1)
         if res is not None:
             bn.update(res=res.ptr, ldr=res.ld)
-        fwd_fields = {k: v for k, v in bn.items() if k not in ("bstats", "coef")}
+        fwd_fields = {k: v for k, v in bn.items() if k not in ("bstats", "coef", "frozen")}
         # ONE op: conv + BN finalize + normalise (+residual) + ReLU — fused into the conv kernel where the layer qualifies
         ops.append(make_op(_lib.OP_CONV_BN, lane=lane, conv=conv_fields, bn=fwd_fields,
-                           barrier=None if lane else self.bn_barrier[c.bn]))
+                           barrier=None if (lane or self.frozen) else self.bn_barrier[c.bn]))
         self.saved[c.name] = dict(src0=src0, src1=src1, up0=up0, raw=raw, act=act, relu=relu, bn=bn, res=res)
         return act
 
@@ -390,9 +408,9 @@ class UnetPlan:
         f1 = self._conv_bn_act(ops, self.stem, self.x8, override=stem_override)
         p1 = T(self, B, f1.H // 2, f1.W // 2, 64)
         self.keep.append(p1.t)
-        self.pool_idx = self._new((B, p1.H, p1.W, 64), torch.uint8) if self.training else None
+        self.pool_idx = self._new((B, p1.H, p1.W, 64), torch.uint8) if self.has_backward else None
         ops.append(make_op(_lib.OP_MAXPOOL_FWD, dtype=self.dtype, B=B, H=f1.H, W=f1.W, C=64, x=f1.ptr, ldx=f1.ld,
-                           y=p1.ptr, ldy=p1.ld, idx=self.pool_idx.data_ptr() if self.training else None))
+                           y=p1.ptr, ldy=p1.ld, idx=self.pool_idx.data_ptr() if self.has_backward else None))
         self.f1, self.p1 = f1, p1
         x = p1
         feats = [f1]
@@ -553,7 +571,8 @@ class UnetPlan:
         else:
             # reduce + apply as ONE op; the apply phase derives its coefficients and writes dgamma / dbeta.  The barrier
             # counter (one-kernel form, opt-in) is cleared by the backward's statistics memset.  Branch lanes: two kernels.
-            bn["barrier"] = None if lane else self.bn_barrier[c.bn] + self.stats.stride(0) * 8
+            # Frozen: one streaming pass (dx does not depend on the reductions) and the finalize, no barrier.
+            bn["barrier"] = None if (lane or self.frozen) else self.bn_barrier[c.bn] + self.stats.stride(0) * 8
             ops.append(make_op(_lib.OP_BN_BWD, lane=lane, **bn))
         return d_raw, g_masked
 
@@ -671,6 +690,13 @@ class UnetPlan:
                                dw=self._gptr(self.stem.name + ".weight")))
         else:
             ops.append(self._wgrad_op(self.stem, self.x8, None, 0, d_r))
+        self.dx_op_index = None
+        if self.want_dx:
+            # the input gradient: the stem's transposed convolution of d_raw, fp32 NCHW (run_backward patches out_nchw)
+            f = dict(dtype=self.dtype, mode=1, src0=d_r.ptr, c0=d_r.C, ld0=d_r.ld, B=B, Hi=d_r.H, Wi=d_r.W, Ho=self.H,
+                     Wo=self.W, kh=7, kw=7, stride=2, pad=3, w=self.w_dgrad[self.stem.name].data_ptr(), Cout=3, out_nchw=None)
+            self.dx_op_index = len(ops)
+            ops.append(make_op(_lib.OP_CONV, **f))
         segs.append(ops)
         return segs
 
@@ -688,11 +714,16 @@ class UnetPlan:
         op_params(self.fwd_ops.array[self.out_op_index]).out_nchw = y.data_ptr()
         self.fwd_ops.run(stream)
 
-    def run_backward(self, dy, stream, after_segment=None):
+    def run_backward(self, dy, stream, after_segment=None, dx=None):
         """Segments run back to back on `stream`; their weight-gradient kernels stay on libd3fk's side stream (no join
         between segments, so the big decoder wgrads overlap the latency-bound encoder segments).  `after_segment(i)`
-        (data-parallel hook) must order its consumer behind BOTH streams; the final join orders `stream` itself."""
+        (data-parallel hook) must order its consumer behind BOTH streams; the final join orders `stream` itself.
+        dx: fp32 NCHW [B,3,H,W] that receives the input gradient (want_dx plans only; required there)."""
         op_params(self.bwd_segments[0].array[self.dy_op_index]).src = dy.data_ptr()
+        if self.want_dx:
+            if dx is None:
+                raise RuntimeError("this plan computes the input gradient: run_backward needs dx")
+            op_params(self.bwd_segments[-1].array[self.dx_op_index]).out_nchw = dx.data_ptr()
         for i, seg in enumerate(self.bwd_segments):
             seg.run(stream, join=False)
             if after_segment is not None:

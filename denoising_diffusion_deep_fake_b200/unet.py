@@ -7,11 +7,18 @@ buffer names (SURVEY Appendix A3) so Lightning checkpoints, `torch.optim.Adam(mo
 `copy.deepcopy` (ema_pytorch) and `.train()/.eval()` keep working.  The arithmetic runs in libd3fk
 (hand-written sm_100a CUDA behind a C ABI); there is no PyTorch/CPU fallback — calling the module
 without the library or off a B200 raises.
+
+Autograd follows nn.Module: a forward with grad enabled and a parameter or the input requiring grad records a graph in BOTH
+modes.  Training mode runs the training plan (batch statistics, running-statistics update); eval mode runs the frozen-BN plan
+(BatchNorm on its running statistics, which nothing updates) — so an eval-mode forward with grad enabled now records a graph
+where it used to return a detached tensor.  Inference callers (the sampler, swap_face, predict_fake, the CLI) run under
+torch.no_grad() and take the fused eval plan as before.  `x.requires_grad` adds the input gradient to the backward.
 """
 import math
 
 import torch
 import torch.nn as nn
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 from .plan import UnetPlan, backward_param_order
@@ -79,7 +86,8 @@ class _Decoder(nn.Module):
 class _UnetFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, module, *params):
-        plan = module._acquire_plan(x, training=True)
+        want_dx = ctx.needs_input_grad[0]
+        plan = module._acquire_plan(x, training=module.training, frozen=not module.training, want_dx=want_dx)
         y = module._run_forward(plan, x)
         ctx.plan, ctx.module = plan, module
         ctx.generation = plan.generation
@@ -88,15 +96,22 @@ class _UnetFunction(torch.autograd.Function):
         return y
 
     @staticmethod
+    @once_differentiable
     def backward(ctx, dy):
         plan, module = ctx.plan, ctx.module
         if plan.generation != ctx.generation:
             raise RuntimeError("d3fk.Unet: the activations of this forward were overwritten by a later forward "
                                "through the same plan before backward() ran")
-        module._run_backward(plan, dy)
+        if plan.frozen and module._dp_hook is not None:
+            raise NotImplementedError("d3fk.Unet: eval-mode (frozen BatchNorm) backward does not run the data-parallel "
+                                      "gradient allreduce; use training mode or disable data parallel")
+        dx = None
+        if plan.want_dx and ctx.needs_input_grad[0]:
+            dx = torch.empty((plan.B, 3, plan.H, plan.W), dtype=torch.float32, device=dy.device)
+        module._run_backward(plan, dy, dx)
         plan.pending_backward = False
         if module.flat_grads:
-            return (None, None) + tuple(None for _ in ctx.names)
+            return (dx, None) + tuple(None for _ in ctx.names)
         flat = module._grad_arena.clone()
         grads = []
         for i, n in enumerate(ctx.names):
@@ -106,7 +121,7 @@ class _UnetFunction(torch.autograd.Function):
             off = module._grad_offsets[n]
             p = module._param_dict[n]
             grads.append(flat[off:off + p.numel()].view(p.shape))
-        return (None, None) + tuple(grads)
+        return (dx, None) + tuple(grads)
 
 
 class Unet(nn.Module):
@@ -219,7 +234,9 @@ class Unet(nn.Module):
             off = self._grad_offsets[n]
             p.grad = self._grad_arena[off:off + p.numel()].view(p.shape)
 
-    def _acquire_plan(self, x, training):
+    def _acquire_plan(self, x, training, frozen=False, want_dx=False):
+        """The cached plan for x's shape and the variant: training, eval (fused, forward only) or, with training=False and
+        frozen=True, the frozen-BN plan; want_dx adds the input gradient to a plan with a backward."""
         if x.dim() != 4 or x.shape[1] != 3:
             raise RuntimeError(f"expected input [B,3,H,W], got {tuple(x.shape)}")
         if x.dtype != torch.float32:
@@ -232,7 +249,10 @@ class Unet(nn.Module):
         if H % 32 != 0 or W % 32 != 0:
             raise RuntimeError(f"Wrong input shape height={H}, width={W}. Expected image height and width "
                                f"divisible by 32.")
-        key = (B, H, W, self.dtype_code, bool(training), dev)
+        frozen = bool(frozen) and not training
+        want_dx = bool(want_dx) and (training or frozen)
+        variant = "train" if training else ("frozen" if frozen else "eval")
+        key = (B, H, W, self.dtype_code, variant, want_dx, dev)
         plans = self._plans.setdefault(key, [])
         plans[:] = [p for p in plans if not p.params_moved()]
         for p in plans:
@@ -248,10 +268,10 @@ class Unet(nn.Module):
         for n, t in list(params.items()) + list(buffers.items()):
             if t.device != dev:
                 raise RuntimeError(f"parameter {n} is on {t.device}, input on {dev}")
-        if training:
+        if training or frozen:
             self._ensure_grad_arena(dev)
         plan = UnetPlan(params, buffers, B, H, W, self.dtype_code, dev, training,
-                        grad_arena=self._grad_arena, grad_offsets=self._grad_offsets)
+                        grad_arena=self._grad_arena, grad_offsets=self._grad_offsets, frozen=frozen, want_dx=want_dx)
         plans.append(plan)
         return plan
 
@@ -293,23 +313,20 @@ class Unet(nn.Module):
         plan.run_forward(x, y, stream)
         return y
 
-    def _run_backward(self, plan, dy):
+    def _run_backward(self, plan, dy, dx=None):
         dy = dy.contiguous()
         stream = torch.cuda.current_stream(dy.device).cuda_stream
         hook = self._dp_hook
-        plan.run_backward(dy, stream, after_segment=(lambda i: hook(i, plan)) if hook is not None else None)
+        plan.run_backward(dy, stream, after_segment=(lambda i: hook(i, plan)) if hook is not None else None, dx=dx)
 
     # -------------------------------------------------------------- nn.Module API
     def forward(self, x):
-        if self.training:
-            if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-                if x.requires_grad:
-                    raise NotImplementedError("d3fk.Unet does not produce input gradients (the reference never "
-                                              "back-propagates into the image)")
-                self._ensure_param_tables()
-                params = [self._param_dict[n] for n in self._param_names]
-                return _UnetFunction.apply(x, self, *params)
-            plan = self._acquire_plan(x, training=True)
-            return self._run_forward(plan, x)
-        plan = self._acquire_plan(x, training=False)
+        """Training mode: batch statistics (running statistics updated).  Eval mode: running statistics.  With grad enabled and
+        a parameter or `x` requiring grad, the call records a graph in either mode (eval mode: the frozen-BN plan; nothing
+        updates the BN buffers); otherwise it runs the plan without autograd (eval mode: the fused eval plan)."""
+        if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
+            self._ensure_param_tables()
+            params = [self._param_dict[n] for n in self._param_names]
+            return _UnetFunction.apply(x, self, *params)
+        plan = self._acquire_plan(x, training=self.training)
         return self._run_forward(plan, x)

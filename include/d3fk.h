@@ -119,14 +119,17 @@ typedef struct d3fk_pack_params {
  * bn_apply with `stats` set finalises the batch statistics itself (mean/invstd/running stats written by block 0)
  * and ignores scale/shift; with stats == NULL it applies the given scale/shift.  bn_bwd_apply derives its
  * coefficients from bstats/mean/invstd/gamma and writes dgamma/dbeta; bn_finalize / bn_bwd_finalize remain as
- * stand-alone entry points. */
+ * stand-alone entry points.  bn_fold with mean / invstd set also writes running_mean and 1/sqrt(running_var + eps) there (the
+ * rows a frozen backward reads). */
 typedef struct d3fk_bn_params {
   int32_t dtype, C, relu;
   int32_t mask_from_x;                  /* backward: ReLU mask = (x*scale + shift > 0) instead of reading `act` — valid when the
                                            forward had no residual (train forward publishes scale / shift for this) */
   int64_t count;                        /* B*H*W */
   const void* x; void* y; const void* res;
-  int32_t ldx, ldy, ldr, _pad1;
+  int32_t ldx, ldy, ldr;
+  int32_t frozen;                       /* backward on the running statistics (eval-mode BN: mean / invstd hold the running values
+                                           BN_FOLD wrote): dx = gamma*invstd*dy', no term from the reductions; dgamma / dbeta as usual */
   double* stats;                        /* [2][C] sum, sumsq of x (from the conv epilogue) */
   const float* gamma; const float* beta;
   float* running_mean; float* running_var; int64_t* num_batches_tracked;
@@ -139,7 +142,7 @@ typedef struct d3fk_bn_params {
   int32_t lddy, ldact, lddx, lddres;
   double* bstats;                       /* [2][C] sum dy', sum dy'*xhat */
   float* dgamma; float* dbeta;
-  float* coef;                          /* [3][C] scratch written by bn_bwd_finalize */
+  float* coef;                          /* [3][C] scratch written by bn_bwd_finalize (nullable) */
   uint32_t* barrier;                    /* D3FK_OP_BN_BWD: zeroed grid-barrier counter (NULL: reduce and apply as two kernels) */
 } d3fk_bn_params;
 
@@ -285,7 +288,8 @@ enum d3fk_op_kind {
   D3FK_OP_SET_SCALARS = 29,   /* scalars params */
   D3FK_OP_JOIN = 30,          /* misc params: n = lane to join back into the main stream */
   D3FK_OP_WGRAD_GROUP = 25,   /* wgrad_group params; forked onto the side streams like D3FK_OP_WGRAD */
-  D3FK_OP_BN_BWD = 24,   /* bn params: bn_bwd_reduce + bn_bwd_apply as one op (one kernel behind a grid barrier when `barrier` is set) */
+  D3FK_OP_BN_BWD = 24,   /* bn params: bn_bwd_reduce + bn_bwd_apply as one op (one kernel behind a grid barrier when `barrier` is set).
+                            frozen: ONE streaming pass writes dx (and dres) and accumulates bstats, then bn_bwd_finalize writes dgamma / dbeta */
   D3FK_OP_NCHW2S2D = 31,   /* layout params (C = 3, cpad = 4, H and W even): fp32 NCHW -> the padded space-to-depth image of conv mode 2:
                               dst[b][h/2][w/2 + 2][((h%2)*2 + (w%2))*4 + c]; the pad pixels / channel are left untouched (zero them once) */
   D3FK_OP_PACK_STEM = 32   /* pack params (Cout, Cin = 3, kh = kw = 7): w_fwd[co][th*64 + tw*16 + (dy*2+dx)*4 + ci] =
