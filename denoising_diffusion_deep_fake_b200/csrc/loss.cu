@@ -198,7 +198,9 @@ __global__ void __launch_bounds__(256, 3) mse_ssim_loss_kernel(d3fk_loss_params 
       if (p.grad) {
         const float xn = (pr - p.lo) * inv_range;
         const float x = fminf(fmaxf(xn, 0.f), 1.f), y = fminf(fmaxf((tg - p.lo) * inv_range, 0.f), 1.f);   // as staged in step 1
-        const float inside = (xn > 0.f && xn < 1.f) ? 1.f : 0.f;   // clip() passes no gradient outside [lo, hi]
+        // torch's clip subgradient: 1 on the closed range [lo, hi] (a prediction exactly at lo or hi keeps its SSIM term),
+        // 0 strictly outside it
+        const float inside = (xn >= 0.f && xn <= 1.f) ? 1.f : 0.f;
         const float dss = A[o] + 2.f * x * Bm[o] + y * Cm[o];
         p.grad[oidx] = k_mse * d - k_ssim * inside * dss;
       }

@@ -261,7 +261,9 @@ typedef struct d3fk_scalars_params {
 /* ---- fused MSE + (1 - SSIM) criterion, forward and gradient
  * (d3f/loss_functions/structural_similarity_loss.py:14-26 + piqa.SSIM defaults, SURVEY Appendix B1).
  * acc[0] += sum (pred-target)^2 ; acc[1] += sum of the SSIM map; the caller zeroes acc and forms
- * loss = (acc[0]/numel + 1 - acc[1]/(B*C*(H-10)*(W-10))) / 2.  grad (nullable) receives grad_scale * dL/dpred. */
+ * loss = (acc[0]/numel + 1 - acc[1]/(B*C*(H-10)*(W-10))) / 2.  grad (nullable) receives grad_scale * dL/dpred, with
+ * torch's clip(0, 1) subgradient on the normalised prediction: the SSIM term passes where lo <= pred <= hi (both ends
+ * included) and is zero strictly outside; the MSE term passes everywhere. */
 typedef struct d3fk_loss_params {
   int32_t B, C, H, W;
   const float* pred; const float* target;   /* fp32 NCHW */
