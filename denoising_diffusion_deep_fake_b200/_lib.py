@@ -90,7 +90,8 @@ class QsampleParams(C.Structure):
 
 class PosteriorParams(C.Structure):
     _fields_ = [("n", i64), ("x", vp), ("x0_hat", vp), ("z", vp), ("coef_table", vp), ("step", vp),
-                ("k_xi", f32), ("k_x0", f32), ("sigma", f32), ("_pad0", f32), ("seed", u64), ("offset", u64)]
+                ("k_xi", f32), ("k_x0", f32), ("sigma", f32), ("r_prev", f32), ("seed", u64), ("offset", u64),
+                ("src", vp), ("mask", vp), ("known_noise", vp), ("chw", i32), ("hw", i32)]
 
 
 class MiscParams(C.Structure):

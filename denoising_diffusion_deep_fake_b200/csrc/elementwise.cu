@@ -873,30 +873,104 @@ __global__ void __launch_bounds__(256) affine_qsample_kernel(d3fk_affine_qsample
   }
 }
 
-// posterior: x = k_xi*x + k_x0*x0_hat + sigma*z
-__global__ void posterior_kernel(d3fk_posterior_params p) {
-  pdl_enter();
-  float k_xi = p.k_xi, k_x0 = p.k_x0, sigma = p.sigma;
-  uint64_t off = p.offset;
+// posterior: x = k_xi*x + k_x0*x0_hat + sigma*z.  The rounding is spelled out (the product k_x0*h rounded, then one fma
+// each for the x and z terms) so the plain and the masked kernel agree bit for bit whatever contraction the compiler would
+// pick in each; it is the contraction the plain kernel has always compiled to.
+__device__ __forceinline__ float posterior1(float k_xi, float x, float k_x0, float h) {
+  return __fmaf_rn(k_xi, x, __fmul_rn(k_x0, h));
+}
+__device__ __forceinline__ float4 posterior4(float k_xi, float4 x, float k_x0, float4 h) {
+  return make_float4(posterior1(k_xi, x.x, k_x0, h.x), posterior1(k_xi, x.y, k_x0, h.y), posterior1(k_xi, x.z, k_x0, h.z),
+                     posterior1(k_xi, x.w, k_x0, h.w));
+}
+__device__ __forceinline__ void posterior_add_noise4(float4& o, float sigma, float4 z) {
+  o.x = __fmaf_rn(sigma, z.x, o.x); o.y = __fmaf_rn(sigma, z.y, o.y);
+  o.z = __fmaf_rn(sigma, z.z, o.z); o.w = __fmaf_rn(sigma, z.w, o.w);
+}
+
+struct PosteriorCoefs {
+  float k_xi, k_x0, sigma, r_prev;
+  uint64_t off;
+};
+__device__ __forceinline__ PosteriorCoefs posterior_coefs(const d3fk_posterior_params& p) {
+  PosteriorCoefs c{p.k_xi, p.k_x0, p.sigma, p.r_prev, p.offset};
   if (p.coef_table) {
     int s = *p.step;
-    k_xi = p.coef_table[4 * s];
-    k_x0 = p.coef_table[4 * s + 1];
-    sigma = p.coef_table[4 * s + 2];
-    off += (uint64_t)s;
+    c.k_xi = p.coef_table[4 * s];
+    c.k_x0 = p.coef_table[4 * s + 1];
+    c.sigma = p.coef_table[4 * s + 2];
+    c.r_prev = p.coef_table[4 * s + 3];
+    c.off += (uint64_t)s;
   }
+  return c;
+}
+
+__global__ void posterior_kernel(d3fk_posterior_params p) {
+  pdl_enter();
+  const PosteriorCoefs c = posterior_coefs(p);
   const long long nvec = p.n / 4;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < nvec; i += (long long)gridDim.x * blockDim.x) {
     float4 x = reinterpret_cast<const float4*>(p.x)[i];
     float4 h = __ldg(reinterpret_cast<const float4*>(p.x0_hat) + i);
-    float4 o = make_float4(k_xi * x.x + k_x0 * h.x, k_xi * x.y + k_x0 * h.y, k_xi * x.z + k_x0 * h.z, k_xi * x.w + k_x0 * h.w);
-    if (sigma != 0.f) {
+    float4 o = posterior4(c.k_xi, x, c.k_x0, h);
+    if (c.sigma != 0.f) {
       float4 z;
       if (p.z) z = __ldg(reinterpret_cast<const float4*>(p.z) + i);
-      else z = philox_normal4(p.seed, (uint64_t)i, off);
-      o.x += sigma * z.x; o.y += sigma * z.y; o.z += sigma * z.z; o.w += sigma * z.w;
+      else z = philox_normal4(p.seed, (uint64_t)i, c.off);
+      posterior_add_noise4(o, c.sigma, z);
     }
     reinterpret_cast<float4*>(p.x)[i] = o;
+  }
+}
+
+__device__ __forceinline__ float composite1(float m, float post, float known) {
+  return __fmaf_rn(m, post, __fmul_rn(1.f - m, known));
+}
+__device__ __forceinline__ float clamp01(float m) { return fminf(fmaxf(m, 0.f), 1.f); }   // NaN -> 0 (keep)
+
+// Masked posterior (replacement inpainting): x = m*post + (1 - m)*known, known = src noised to r_prev (d3fk.h).
+// blockIdx.y = sample; a thread owns the 4-element vector i = b*chw/4 + v of one channel row, exactly the vector
+// posterior_kernel owns (same z counter), and reads its 4 pixels' mask (the C channels of a pixel read the same mask
+// vector; after the first it comes from L2).  A vector whose 4 mask values are all 1 reads no src and draws no n; all 0
+// reads no x / x0_hat and draws no z — with a hard mask each pixel costs the bytes of only one of the two updates.
+__global__ void __launch_bounds__(256) posterior_masked_kernel(d3fk_posterior_params p) {
+  pdl_enter();
+  const PosteriorCoefs c = posterior_coefs(p);
+  const float a = sqrtf(1.f - c.r_prev), s = sqrtf(c.r_prev);
+  const int b = blockIdx.y;
+  const unsigned vpp = (unsigned)p.hw / 4u, vps = (unsigned)p.chw / 4u;
+  const long long base = (long long)b * vps;
+  const float4* mask = reinterpret_cast<const float4*>(p.mask) + (long long)b * vpp;
+  for (unsigned v = blockIdx.x * blockDim.x + threadIdx.x; v < vps; v += gridDim.x * blockDim.x) {
+    float4 m = __ldg(mask + v % vpp);
+    m = make_float4(clamp01(m.x), clamp01(m.y), clamp01(m.z), clamp01(m.w));
+    const bool all1 = m.x == 1.f && m.y == 1.f && m.z == 1.f && m.w == 1.f;
+    const bool all0 = m.x == 0.f && m.y == 0.f && m.z == 0.f && m.w == 0.f;
+    const long long i = base + v;
+    float4 post = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (!all0) {
+      float4 x = reinterpret_cast<const float4*>(p.x)[i];
+      float4 h = __ldg(reinterpret_cast<const float4*>(p.x0_hat) + i);
+      post = posterior4(c.k_xi, x, c.k_x0, h);
+      if (c.sigma != 0.f) {
+        float4 z;
+        if (p.z) z = __ldg(reinterpret_cast<const float4*>(p.z) + i);
+        else z = philox_normal4(p.seed, (uint64_t)i, c.off);
+        posterior_add_noise4(post, c.sigma, z);
+      }
+    }
+    float4 known = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (!all1) {
+      float4 n = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (c.r_prev != 0.f) {
+        if (p.known_noise) n = __ldg(reinterpret_cast<const float4*>(p.known_noise) + i);
+        else n = philox_normal4(p.seed, (uint64_t)i | (1ull << 63), c.off);
+      }
+      float4 x = __ldg(reinterpret_cast<const float4*>(p.src) + i);
+      known = make_float4(blend1(a, x.x, s, n.x), blend1(a, x.y, s, n.y), blend1(a, x.z, s, n.z), blend1(a, x.w, s, n.w));
+    }
+    reinterpret_cast<float4*>(p.x)[i] = make_float4(composite1(m.x, post.x, known.x), composite1(m.y, post.y, known.y),
+                                                    composite1(m.z, post.z, known.z), composite1(m.w, post.w, known.w));
   }
 }
 
@@ -1301,7 +1375,18 @@ int launch_affine_qsample(const d3fk_affine_qsample_params* p, cudaStream_t s) {
 }
 int launch_posterior(const d3fk_posterior_params* p, cudaStream_t s) {
   D3FK_CHECK_ARG(p->n % 4 == 0, "n must be a multiple of 4");
-  launch_k(posterior_kernel, dim3(grid_for(p->n / 4, 256)), dim3(256), 0, s, dim3(1, 1, 1), *p);
+  if (!p->mask) {
+    launch_k(posterior_kernel, dim3(grid_for(p->n / 4, 256)), dim3(256), 0, s, dim3(1, 1, 1), *p);
+    count_launch();
+    return check_launch("posterior_step");
+  }
+  D3FK_CHECK_ARG(p->src && p->x && p->x0_hat, "the masked posterior needs x, x0_hat and src");
+  D3FK_CHECK_ARG(p->hw > 0 && p->hw % 4 == 0 && p->chw >= p->hw && p->chw % p->hw == 0, "hw must be a multiple of 4 dividing chw");
+  D3FK_CHECK_ARG(p->n > 0 && p->n % p->chw == 0 && p->n / p->chw <= 65535, "n must be 1..65535 samples of chw elements");
+  D3FK_CHECK_ARG((((uintptr_t)p->x | (uintptr_t)p->x0_hat | (uintptr_t)p->src | (uintptr_t)p->mask | (uintptr_t)p->z |
+                   (uintptr_t)p->known_noise) & 15) == 0, "buffers must be 16-byte aligned");
+  const int gx = cdiv(p->chw / 4, 256);           // one 4-element vector per thread
+  launch_k(posterior_masked_kernel, dim3(gx, (unsigned)(p->n / p->chw)), dim3(256), 0, s, dim3(1, 1, 1), *p);
   count_launch();
   return check_launch("posterior_step");
 }

@@ -24,6 +24,12 @@ def _require_cuda_f32(t, name):
     _lib.init(t.device.index)
 
 
+def composite_(out, src, mask):
+    """In place: out = m*out + (1 - m)*src (mask as normalize_mask accepts) — the masked posterior of the last step, whose
+    known region is the source itself; exactly src where m == 0 and out where m == 1."""
+    return posterior_step_(out, out, 0.0, 0.0, src=src, mask=mask)
+
+
 def q_sample(batch, lam, noise=None, y=None, seed=0, offset=0, fixed_r=None, return_aux=False, out=None):
     """noisy = sqrt(1-r)*batch + sqrt(r)*noise with per-sample r = 1/lam*log(1/(y(1-c)+c)), c = e^-lam.
     noise / y: optional tensors (parity with the reference's torch.randn_like / torch.rand draws);
@@ -71,15 +77,75 @@ def posterior_coeffs(r_i, r_prev, eta):
     return k_xi, k_x0, sigma
 
 
-def posterior_step_(x_i, x0_hat, r_i, r_prev, z=None, eta=0.0, seed=0, offset=0):
-    """In-place posterior update of x_i (one fused kernel)."""
+def posterior_coef_table(grid, eta):
+    """Rows (k_xi, k_x0, sigma, r_prev) of the sampler's device coefficient table, one per step i from grid[i] to
+    grid[i + 1].  A step from ratio 0 returns x0_hat (the single-pass case); r_prev is the ratio the masked update noises
+    the source to (0 at the last step: the known region is the source itself)."""
+    rows = []
+    for i in range(len(grid) - 1):
+        if grid[i] <= 0.0:
+            rows.append((0.0, 1.0, 0.0, 0.0))
+        else:
+            rows.append(posterior_coeffs(grid[i], grid[i + 1], eta) + (max(float(grid[i + 1]), 0.0),))
+    return rows
+
+
+def normalize_mask(mask, batch, height, width):
+    """An inpainting mask as the contiguous float32 [B,1,H,W] buffer the masked posterior reads (1 = generate, 0 = keep,
+    fractions feather; the kernel clamps to [0, 1]).  Accepts [H,W], [1,1,H,W] or [B,1,H,W], float32 or bool, on any
+    device (the result stays there)."""
+    if not torch.is_tensor(mask):
+        raise TypeError(f"mask must be a torch tensor, got {type(mask).__name__}")
+    if mask.dtype not in (torch.float32, torch.bool):
+        raise TypeError(f"mask must be float32 or bool, got {mask.dtype}")
+    shape = tuple(mask.shape)
+    if shape not in ((height, width), (1, 1, height, width), (batch, 1, height, width)):
+        raise ValueError(f"mask of shape {shape} does not broadcast to [{batch},1,{height},{width}]: "
+                         f"give [H,W], [1,1,H,W] or [B,1,H,W]")
+    return mask.reshape(-1, 1, height, width).expand(batch, 1, height, width).to(torch.float32).contiguous()
+
+
+def posterior_step_(x_i, x0_hat, r_i, r_prev, z=None, eta=0.0, seed=0, offset=0, src=None, mask=None, known_noise=None):
+    """In-place posterior update of x_i (one fused kernel).
+    With `mask` (see normalize_mask) and `src` ([B,3,H,W] like x_i): x_i = m*post + (1 - m)*known, known = src noised to
+    r_prev = sqrt(1 - r_prev)*src + sqrt(r_prev)*known_noise — replacement inpainting; where m == 0 the result is
+    q_sample(src, fixed_r=r_prev, noise=known_noise) bit for bit, src itself at r_prev = 0.  known_noise=None draws it
+    in-kernel from its own Philox stream of (seed, offset).  x0_hat may be x_i itself."""
     _require_cuda_f32(x_i, "x_i")
     if not x_i.is_contiguous() or not x0_hat.is_contiguous():
         raise ValueError("posterior_step_ needs contiguous tensors")
     k_xi, k_x0, sigma = posterior_coeffs(float(r_i), float(r_prev), eta)
+    masked = {}
+    if mask is None:
+        if src is not None or known_noise is not None:
+            raise ValueError("posterior_step_: src and known_noise are the masked update's inputs; give a mask with them")
+    else:
+        if x_i.dim() != 4:
+            raise ValueError(f"the masked posterior needs x_i of shape [B,C,H,W], got {tuple(x_i.shape)}")
+        B, _, H, W = x_i.shape
+        r_prev_k = max(float(r_prev), 0.0)
+        if r_prev_k > 1.0:
+            raise ValueError(f"r_prev must lie in [0, 1], got {r_prev}")
+        if src is None:
+            raise ValueError("posterior_step_: a mask needs the source image `src`")
+        for name, t in (("src", src), ("known_noise", known_noise)):
+            if t is None:
+                continue
+            if t.dtype != torch.float32:
+                raise TypeError(f"{name} must be float32, got {t.dtype}")
+            if t.shape != x_i.shape or t.device != x_i.device:
+                raise ValueError(f"{name} must have x_i's shape {tuple(x_i.shape)} and device {x_i.device}, "
+                                 f"got {tuple(t.shape)} on {t.device}")
+        if mask.device != x_i.device:
+            raise ValueError(f"mask must be on {x_i.device}, got {mask.device}")
+        src = src.contiguous()
+        mask = normalize_mask(mask, B, H, W)
+        known_noise = None if known_noise is None else known_noise.contiguous()
+        masked = dict(r_prev=r_prev_k, src=src.data_ptr(), mask=mask.data_ptr(),
+                      known_noise=None if known_noise is None else known_noise.data_ptr(), chw=x_i[0].numel(), hw=H * W)
     op = make_op(_lib.OP_POSTERIOR, n=x_i.numel(), x=x_i.data_ptr(), x0_hat=x0_hat.data_ptr(),
                  z=None if z is None else z.contiguous().data_ptr(), k_xi=k_xi, k_x0=k_x0, sigma=sigma,
-                 seed=int(seed), offset=int(offset))
+                 seed=int(seed), offset=int(offset), **masked)
     _lib.run_single(op, _stream(x_i))
     return x_i
 

@@ -214,10 +214,17 @@ def modify(config_path, checkpoint_path, synthetic, size, checkpoint_dir):
 @click.option("--r_start", type=float, default=1.0, help="noise ratio to start from (1 = pure noise)")
 @click.option("--seed", type=int, default=0)
 @click.option("--out", default="samples.pt")
-def sample(checkpoint_path, which, steps, batch, size, eta, r_start, seed, out):
-    """Iterative reverse-diffusion sampling with CUDA-graph replayed steps (new entry point)."""
+@click.option("--source", default=None, help="torch.save'd normalised images [B,3,H,W] to inpaint (needs --mask; "
+              "sets the batch and size)")
+@click.option("--mask", default=None, help="torch.save'd mask [H,W], [1,1,H,W] or [B,1,H,W]: 1 = generate, 0 = keep "
+              "the source, fractions feather")
+def sample(checkpoint_path, which, steps, batch, size, eta, r_start, seed, out, source, mask):
+    """Iterative reverse-diffusion sampling with CUDA-graph replayed steps (new entry point).  With --source and --mask
+    the sampler regenerates only the masked region and keeps the source outside it (masked face swap)."""
     from .sampler import Sampler
     from .unet import Unet
+    if (source is None) != (mask is None):
+        raise click.UsageError("--source and --mask go together")
     dev = torch.device("cuda", torch.cuda.current_device())
     if checkpoint_path:
         try:
@@ -229,8 +236,16 @@ def sample(checkpoint_path, which, steps, batch, size, eta, r_start, seed, out):
     else:
         model = Unet()
     model = model.to(dev).eval()
-    smp = Sampler(model, batch, size, size, steps, r_start=r_start, eta=eta, seed=seed)
-    x0 = smp.run()
+    if source is None:
+        smp = Sampler(model, batch, size, size, steps, r_start=r_start, eta=eta, seed=seed)
+        x0 = smp.run()
+    else:
+        src = torch.load(source, map_location="cpu").to(dev, torch.float32).contiguous()
+        if src.dim() != 4 or src.shape[1] != 3:
+            raise click.UsageError(f"--source must hold [B,3,H,W] images, got {tuple(src.shape)}")
+        B, _, H, W = src.shape
+        smp = Sampler(model, B, H, W, steps, r_start=r_start, eta=eta, seed=seed, masked=True)
+        x0 = smp.run(src=src, mask=torch.load(mask, map_location="cpu"))
     torch.save(x0.cpu(), out)
     print(f"wrote {tuple(x0.shape)} samples to {out}")
 

@@ -12,19 +12,23 @@ Chains (opt-in, `chains=` / D3FK_SAMPLER_CHAINS): in eval mode the images of a b
 affine), so the batch can be split into sub-batches, each with its own plan, step counter and CUDA stream, captured as
 parallel branches of the same graph.  Measured on B200 at B=64 @128x128 this LOSES (1.11 ms/step with one chain, 1.18 with
 two, 1.43 with four): the forward is bound by kernel throughput, not by launch latency, and smaller sub-batches only add
-per-kernel fixed cost.  It pays only for small batches of large images sharing one GPU; default 1."""
+per-kernel fixed cost.  It pays only for small batches of large images sharing one GPU; default 1.
+
+Masked sampling (`masked=True`; replacement inpainting, as RePaint without resampling): every step blends the update with
+the source noised to the step's target ratio, x = m*post + (1 - m)*known, inside the same posterior kernel — the mask
+adds no launch.  At the last step known is the source itself, so where the mask is 0 the result is the source exactly."""
 import os
 
 import torch
 
 from . import _lib
 from ._lib import make_op, op_params
-from .functional import noise_ratio_grid, posterior_coeffs, posterior_step_, q_sample
+from .functional import composite_, noise_ratio_grid, normalize_mask, posterior_coef_table, posterior_step_, q_sample
 
 
 class Sampler:
     def __init__(self, model, batch, height, width, n_steps, r_start=1.0, eta=0.0, seed=0, use_graph=True,
-                 steps_per_graph=1, chains=None):
+                 steps_per_graph=1, chains=None, masked=False):
         p = next(model.parameters())
         if not p.is_cuda:
             raise _lib.D3fkError("Sampler needs the model on a B200 (sm_100a) CUDA device")
@@ -39,13 +43,12 @@ class Sampler:
         self.plan = model._acquire_plan(self.x, training=False)
         self.plan.pending_backward = True        # reserve this plan instance for the sampler
         model.train(was_training)
-        coefs = []
-        for i in range(n_steps):
-            if self.grid[i] <= 0.0:
-                coefs.append((0.0, 1.0, 0.0, 0.0))
-            else:
-                coefs.append(posterior_coeffs(self.grid[i], self.grid[i + 1], eta) + (0.0,))
-        self.coef_table = torch.tensor(coefs, dtype=torch.float32, device=self.device).contiguous()
+        self.coef_table = torch.tensor(posterior_coef_table(self.grid, eta), dtype=torch.float32,
+                                       device=self.device).contiguous()
+        self.masked = bool(masked)
+        # the source and mask buffers the masked posterior ops point at (run() copies its inputs into them)
+        self.src = torch.zeros_like(self.x) if self.masked else None
+        self.mask = torch.zeros(batch, 1, height, width, dtype=torch.float32, device=self.device) if self.masked else None
         self.step = torch.zeros(1, dtype=torch.int32, device=self.device)
         if chains is None:
             chains = int(os.environ.get("D3FK_SAMPLER_CHAINS", "1"))
@@ -63,10 +66,14 @@ class Sampler:
             ops = list(plan.fwd_ops)
             op_params(ops[plan.in_op_index]).src = xs.data_ptr()
             op_params(ops[plan.out_op_index]).out_nchw = hs.data_ptr()
+            masked = {}
+            if self.masked:
+                masked = dict(src=self.src[c * b:(c + 1) * b].data_ptr(), mask=self.mask[c * b:(c + 1) * b].data_ptr(),
+                              chw=3 * height * width, hw=height * width)
             # independent Philox streams per chain (the kernel's counter is the element index within its own sub-batch)
             ops.append(make_op(_lib.OP_POSTERIOR, n=xs.numel(), x=xs.data_ptr(), x0_hat=hs.data_ptr(),
                                coef_table=self.coef_table.data_ptr(), step=step.data_ptr(),
-                               seed=self.seed + 0x9E3779B1 * c, offset=0))
+                               seed=self.seed + 0x9E3779B1 * c, offset=0, **masked))
             ops.append(make_op(_lib.OP_INC, p0=step.data_ptr(), n=1))
             self.kernels_per_step += len(ops)
             self.chain_plans.append(plan)
@@ -111,23 +118,41 @@ class Sampler:
         self.graph = g
 
     @torch.no_grad()
-    def run(self, x_start=None, noises=None):
+    def run(self, x_start=None, noises=None, src=None, mask=None, known_noises=None):
         """x_start: state at ratio r_start ([B,3,H,W] fp32; default: Philox N(0,1) when r_start == 1).
-        noises: optional [n_steps,B,3,H,W] (eta > 0 parity runs; forces the eager path).  Returns x_0."""
+        noises: optional [n_steps,B,3,H,W] (eta > 0 parity runs; forces the eager path).  Returns x_0.
+        Masked sampler: src [B,3,H,W] (the image to keep outside the mask) and mask (see functional.normalize_mask) are
+        required; x_start defaults to src noised to r_start (Philox N(0,1) at r_start == 1, as unmasked).  known_noises:
+        optional [n_steps,B,3,H,W], the noise of the known region at each step (forces the eager path, as noises does; the
+        eager path otherwise draws the graph's in-kernel known noise)."""
+        if self.masked != (src is not None and mask is not None) or (not self.masked and known_noises is not None):
+            raise ValueError("a masked Sampler needs src and mask (and an unmasked one takes neither, nor known_noises)")
+        eager = noises is not None or known_noises is not None
         self.refresh_weights()
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        if self.use_graph and self.graph is None and noises is None:
+        if self.use_graph and self.graph is None and not eager:
             self._capture()                      # (its warm-up launch scribbles on self.x: capture first)
+        if self.masked:
+            self.src.copy_(src)
+            self.mask.copy_(normalize_mask(mask, self.B, self.H, self.W))
         if x_start is None:
-            zeros = torch.zeros_like(self.x)
-            self.x.copy_(q_sample(zeros, 1.0, seed=self.seed ^ 0x5EED, fixed_r=1.0))
+            # (q_sample at ratio 1 is the noise alone: the masked start at r_start == 1 is the unmasked one)
+            base = self.src if self.masked else torch.zeros_like(self.x)
+            r0 = max(self.r_start, 0.0) if self.masked else 1.0
+            self.x.copy_(q_sample(base, 1.0, seed=self.seed ^ 0x5EED, fixed_r=r0))
         else:
             self.x.copy_(x_start)
-        if noises is not None:
+        if eager:
             for i in range(self.n_steps):
                 self.plan.run_forward(self.x, self.x0_hat, stream)
-                posterior_step_(self.x, self.x0_hat, self.grid[i], self.grid[i + 1] if self.grid[i] > 0 else 0.0,
-                                z=noises[i], eta=self.eta)
+                r_prev = self.grid[i + 1] if self.grid[i] > 0 else 0.0
+                z = None if noises is None else noises[i]
+                if self.masked:
+                    posterior_step_(self.x, self.x0_hat, self.grid[i], r_prev, z=z, eta=self.eta, seed=self.seed,
+                                    offset=i, src=self.src, mask=self.mask,
+                                    known_noise=None if known_noises is None else known_noises[i])
+                else:
+                    posterior_step_(self.x, self.x0_hat, self.grid[i], r_prev, z=z, eta=self.eta)
             return self.x.clone()
         for st in self.chain_steps:
             st.zero_()
@@ -149,17 +174,26 @@ def sample(model, x_start, n_steps, r_start=1.0, eta=0.0, seed=0, noises=None, u
 
 
 @torch.no_grad()
-def swap_face(model, real, n_steps=1, r_start=0.0, eta=0.0, seed=0):
+def swap_face(model, real, n_steps=1, r_start=0.0, eta=0.0, seed=0, mask=None):
     """Push `real` (identity A, normalised to [-1,1]) toward the identity `model` was trained on.
     n_steps=1, r_start=0 reproduces the reference exactly: fake = model(real)
     (d3f/train_deep_fake/lit_module.py:189,266).  r_start>0 noises the source to that ratio first and
-    runs the iterative sampler from there."""
+    runs the iterative sampler from there.
+    mask ([H,W], [1,1,H,W] or [B,1,H,W]; 1 = swap, 0 = keep `real`, fractions feather): r_start <= 0 gives the composite
+    m*model(real) + (1 - m)*real; r_start > 0 runs the masked sampler, which keeps the source outside the mask at every
+    step, so the swapped region is generated in context.  Where m == 0 the result is `real` exactly."""
     if r_start <= 0.0:
         was = model.training
         model.eval()
         out = model(real)
         model.train(was)
-        return out
+        if mask is None:
+            return out
+        B, _, H, W = real.shape
+        return composite_(out, real, normalize_mask(mask, B, H, W).to(out.device))
+    if mask is not None:
+        B, _, H, W = real.shape
+        return Sampler(model, B, H, W, n_steps, r_start, eta, seed, masked=True).run(src=real, mask=mask)
     # the start noise comes from a Philox key of its own (as Sampler.run's does): with the sampler's key the first ancestral
     # z (eta > 0; posterior step 0 draws philox(seed, element, offset 0)) would be the very noise the source was noised with
     x_start = q_sample(real, 1.0, seed=seed ^ 0x5EED, fixed_r=r_start)

@@ -703,30 +703,49 @@ class DeepFakeModule(nn.Module):
             set_lr(o, lr)
 
     @torch.no_grad()
-    def predict_fake(self, real, model_a_or_b):
+    def predict_fake(self, real, model_a_or_b, mask=None):
         """predict_fake (lit_module.py:251-270).  Two input forms:
         * the reference's: one uint8 BGR frame [H,W,3] (numpy, as cv2 delivers it) or a batch [N,H,W,3] (numpy or a uint8
           CUDA tensor) -> the fake frame(s), same type and layout.  Normalisation, the network and the conversion back
           all run on the device (d3fk_frames_to_tensor / d3fk_tensor_to_frames); model "a" uses mean_b / std_b and
           model "b" mean_a / std_a, as the reference does (:253-257).
-        * a normalised fp32 tensor [B,3,H,W] -> the network output (tensor-level use inside training code)."""
+        * a normalised fp32 tensor [B,3,H,W] -> the network output (tensor-level use inside training code).
+        mask (optional; 1 = swap, 0 = keep the input, fractions feather): the output is m*fake + (1 - m)*input, fused into
+        one kernel after the network.  Any form functional.normalize_mask takes; with uint8 frames also a uint8 [H,W] or
+        [N,H,W] mask in 0..255 (numpy or torch, as cv2 produces masks), scaled by 1/255.  Where m == 0 the output frame
+        is the input's own round trip through normalisation, tensor_to_frames(frames_to_tensor(frame))."""
         import numpy as np
-        from .functional import frames_to_tensor, tensor_to_frames
+        from .functional import composite_, frames_to_tensor, normalize_mask, tensor_to_frames
         model = self.model_a if model_a_or_b == "a" else self.model_b
         is_numpy = isinstance(real, np.ndarray)
         frames = torch.from_numpy(np.ascontiguousarray(real)) if is_numpy else real
+        if isinstance(mask, np.ndarray):
+            mask = torch.from_numpy(np.ascontiguousarray(mask))
+        if mask is not None and mask.dtype == torch.uint8:
+            if frames.dtype != torch.uint8:
+                raise TypeError("a uint8 mask goes with uint8 frames; give a float32 or bool mask for a normalised tensor")
+            if mask.dim() == 3:
+                mask = mask.unsqueeze(1)                 # [N,H,W] -> [N,1,H,W]
+            mask = mask.to(torch.float32) / 255.0
+
+        def composited(out, x):
+            if mask is None:
+                return out
+            B, _, H, W = x.shape
+            return composite_(out, x, normalize_mask(mask, B, H, W).to(out.device))
+
         was = model.training
         model.eval()
         try:
             if frames.dtype != torch.uint8:
-                return model(frames)
+                return composited(model(frames), frames)
             p = self.hparams
             other = "b" if model_a_or_b == "a" else "a"
             mean, std = p.get(f"mean_{other}", [0.5] * 3), p.get(f"std_{other}", [0.5] * 3)
             single = frames.dim() == 3
             dev = next(model.parameters()).device
             x = frames_to_tensor(frames.to(dev, non_blocking=True), mean, std)
-            fake = tensor_to_frames(model(x), mean, std)
+            fake = tensor_to_frames(composited(model(x), x), mean, std)
             fake = fake[0] if single else fake
             return fake.cpu().numpy() if is_numpy else fake
         finally:

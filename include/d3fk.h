@@ -227,14 +227,24 @@ typedef struct d3fk_affine_qsample_params {
 } d3fk_affine_qsample_params;
 
 /* ---- posterior update x_{i-1} = k_xi*x_i + k_x0*x0_hat + sigma*z (SURVEY §8a row S) ------------
- * Coefficients come from coef_table[*step][0..2] when coef_table is set (CUDA-graph replay: the
- * graph is step-independent), else from the immediates. z supplied or Philox(seed, offset+*step). */
+ * Coefficients come from coef_table[*step][0..3] = (k_xi, k_x0, sigma, r_prev) when coef_table is set (CUDA-graph
+ * replay: the graph is step-independent), else from the immediates. z supplied or Philox(seed, offset+*step): counter
+ * (i, i >> 32, off, off >> 32) for the 4-element vector i of the op's (sub-)batch.
+ * Masked form (mask != NULL; replacement inpainting): x is NCHW with chw = C*H*W elements per sample and hw = H*W, src
+ * has x's shape and mask is [B][H][W] (broadcast over channels, clamped to [0, 1]; 1 = generate, 0 = keep):
+ *   known = sqrt(1 - r_prev)*src + sqrt(r_prev)*n      (rounded as d3fk_q_sample with fixed_r = r_prev: known == src at 0)
+ *   x     = m*post + (1 - m)*known                      (fma(m, post, (1 - m)*known): exactly post at m = 1, known at 0)
+ * n is known_noise when supplied, else drawn in-kernel from a stream no other draw uses: the key and offset of z with
+ * bit 31 set in counter word 1, i.e. counter (i, (i >> 32) | 0x80000000, off, off >> 32).  z is the unmasked kernel's, so
+ * a mask of ones reproduces the unmasked update bit for bit.  x0_hat may alias x. */
 typedef struct d3fk_posterior_params {
   int64_t n;
   float* x; const float* x0_hat; const float* z;
   const float* coef_table; const int32_t* step;
-  float k_xi, k_x0, sigma, _pad0;
+  float k_xi, k_x0, sigma, r_prev;
   uint64_t seed, offset;
+  const float* src; const float* mask; const float* known_noise;   /* masked form: all NULL for the plain update */
+  int32_t chw, hw;
 } d3fk_posterior_params;
 
 typedef struct d3fk_misc_params {          /* MEMSET: p0[0..n) bytes = 0; INC: *(int32*)p0 += 1; PACK_ALL: see enum */
