@@ -94,6 +94,10 @@ class PosteriorParams(C.Structure):
                 ("src", vp), ("mask", vp), ("known_noise", vp), ("chw", i32), ("hw", i32)]
 
 
+class Posterior2mParams(C.Structure):
+    _fields_ = [("base", PosteriorParams), ("x0_prev", vp), ("c", f32), ("_pad", i32)]
+
+
 class MiscParams(C.Structure):
     _fields_ = [("p0", vp), ("n", i64)]
 
@@ -128,7 +132,7 @@ class _OpUnion(C.Union):
                 ("qsample", QsampleParams), ("posterior", PosteriorParams), ("misc", MiscParams),
                 ("adam", AdamParams), ("loss", LossParams), ("convbn", ConvBnParams), ("upcat", UpcatParams),
                 ("wgrad_group", WgradGroupParams), ("frames", FramesParams),
-                ("affine_qsample", AffineQsampleParams), ("scalars", ScalarsParams)]
+                ("affine_qsample", AffineQsampleParams), ("scalars", ScalarsParams), ("posterior_2m", Posterior2mParams)]
 
 
 class Op(C.Structure):
@@ -140,7 +144,7 @@ class Op(C.Structure):
  OP_BN_BWD_FINALIZE, OP_BN_BWD_APPLY, OP_MAXPOOL_FWD, OP_MAXPOOL_BWD, OP_SUMPOOL2, OP_CHANSUM, OP_QSAMPLE,
  OP_POSTERIOR, OP_MEMSET, OP_INC, OP_ADAM, OP_PACK_ALL, OP_LOSS, OP_CONV_BN, OP_UPCAT, OP_BN_BWD, OP_WGRAD_GROUP, OP_FRAMES_TO_TENSOR, OP_TENSOR_TO_FRAMES,
  OP_AFFINE_QSAMPLE, OP_SET_SCALARS, OP_JOIN) = range(1, 31)
-OP_NCHW2S2D, OP_PACK_STEM = 31, 32
+OP_NCHW2S2D, OP_PACK_STEM, OP_POSTERIOR_2M = 31, 32, 33
 MAX_LANES = 2
 
 _UNION_FIELD = {OP_CONV: "conv", OP_WGRAD: "wgrad", OP_PACK: "pack", OP_NCHW2NHWC: "layout",
@@ -151,12 +155,13 @@ _UNION_FIELD = {OP_CONV: "conv", OP_WGRAD: "wgrad", OP_PACK: "pack", OP_NCHW2NHW
                 OP_LOSS: "loss", OP_CONV_BN: "convbn", OP_UPCAT: "upcat", OP_BN_BWD: "bn",
                 OP_WGRAD_GROUP: "wgrad_group", OP_FRAMES_TO_TENSOR: "frames", OP_TENSOR_TO_FRAMES: "frames",
                 OP_AFFINE_QSAMPLE: "affine_qsample", OP_SET_SCALARS: "scalars", OP_JOIN: "misc",
-                OP_NCHW2S2D: "layout", OP_PACK_STEM: "pack"}
+                OP_NCHW2S2D: "layout", OP_PACK_STEM: "pack", OP_POSTERIOR_2M: "posterior_2m"}
 _PARAM_CLS = {"conv": ConvParams, "wgrad": WgradParams, "pack": PackParams, "bn": BnParams, "pool": PoolParams,
               "layout": LayoutParams, "chansum": ChansumParams, "qsample": QsampleParams,
               "posterior": PosteriorParams, "misc": MiscParams, "adam": AdamParams, "loss": LossParams,
               "convbn": ConvBnParams, "upcat": UpcatParams, "wgrad_group": WgradGroupParams,
-              "frames": FramesParams, "affine_qsample": AffineQsampleParams, "scalars": ScalarsParams}
+              "frames": FramesParams, "affine_qsample": AffineQsampleParams, "scalars": ScalarsParams,
+              "posterior_2m": Posterior2mParams}
 
 SINGLE_ENTRY = {OP_CONV: "d3fk_conv", OP_WGRAD: "d3fk_wgrad", OP_PACK: "d3fk_pack_weights",
                 OP_NCHW2NHWC: "d3fk_nchw_to_nhwc", OP_BN_FINALIZE: "d3fk_bn_finalize", OP_BN_APPLY: "d3fk_bn_apply",
@@ -167,7 +172,7 @@ SINGLE_ENTRY = {OP_CONV: "d3fk_conv", OP_WGRAD: "d3fk_wgrad", OP_PACK: "d3fk_pac
                 OP_ADAM: "d3fk_adam", OP_LOSS: "d3fk_mse_ssim_loss", OP_CONV_BN: "d3fk_conv_bn", OP_UPCAT: "d3fk_upcat", OP_BN_BWD: "d3fk_bn_bwd",
                 OP_WGRAD_GROUP: "d3fk_wgrad_group", OP_FRAMES_TO_TENSOR: "d3fk_frames_to_tensor",
                 OP_TENSOR_TO_FRAMES: "d3fk_tensor_to_frames", OP_AFFINE_QSAMPLE: "d3fk_affine_q_sample",
-                OP_SET_SCALARS: "d3fk_set_scalars"}
+                OP_SET_SCALARS: "d3fk_set_scalars", OP_POSTERIOR_2M: "d3fk_posterior_2m_step"}
 EXPORTS = ["d3fk_version", "d3fk_sizeof_op", "d3fk_init", "d3fk_last_error", "d3fk_device_error_flag", "d3fk_run",
            "d3fk_run_nojoin", "d3fk_side_stream_join", "d3fk_run_profile", "d3fk_launch_count", "d3fk_debug_timeline"] + sorted(set(SINGLE_ENTRY.values()))
 

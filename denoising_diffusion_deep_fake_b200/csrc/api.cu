@@ -59,6 +59,7 @@ int launch_tensor_to_frames(const d3fk_frames_params*, cudaStream_t);
 int launch_affine_qsample(const d3fk_affine_qsample_params*, cudaStream_t);
 int launch_qsample(const d3fk_qsample_params*, cudaStream_t);
 int launch_posterior(const d3fk_posterior_params*, cudaStream_t);
+int launch_posterior_2m(const d3fk_posterior_2m_params*, cudaStream_t);
 int launch_inc(const d3fk_misc_params*, cudaStream_t);
 int launch_adam(const d3fk_adam_params*, cudaStream_t);
 int launch_set_scalars(const d3fk_scalars_params*, cudaStream_t);
@@ -134,6 +135,7 @@ static int run_one(const d3fk_op* op, cudaStream_t s) {
     case D3FK_OP_AFFINE_QSAMPLE: return launch_affine_qsample(&op->u.affine_qsample, s);
     case D3FK_OP_QSAMPLE: return launch_qsample(&op->u.qsample, s);
     case D3FK_OP_POSTERIOR: return launch_posterior(&op->u.posterior, s);
+    case D3FK_OP_POSTERIOR_2M: return launch_posterior_2m(&op->u.posterior_2m, s);
     case D3FK_OP_MEMSET: {
       cudaError_t e = cudaMemsetAsync(op->u.misc.p0, 0, (size_t)op->u.misc.n, s);
       if (e != cudaSuccess) return set_error(D3FK_ERR_CUDA, "memset: %s", cudaGetErrorString(e));
@@ -399,6 +401,7 @@ SINGLE(d3fk_tensor_to_frames, d3fk_frames_params, launch_tensor_to_frames)
 SINGLE(d3fk_affine_q_sample, d3fk_affine_qsample_params, launch_affine_qsample)
 SINGLE(d3fk_q_sample, d3fk_qsample_params, launch_qsample)
 SINGLE(d3fk_posterior_step, d3fk_posterior_params, launch_posterior)
+SINGLE(d3fk_posterior_2m_step, d3fk_posterior_2m_params, launch_posterior_2m)
 SINGLE(d3fk_adam, d3fk_adam_params, launch_adam)
 SINGLE(d3fk_set_scalars, d3fk_scalars_params, launch_set_scalars)
 SINGLE(d3fk_mse_ssim_loss, d3fk_loss_params, launch_loss)

@@ -974,6 +974,107 @@ __global__ void __launch_bounds__(256) posterior_masked_kernel(d3fk_posterior_pa
   }
 }
 
+// Second-order multistep (DPM-Solver++ 2M) posterior, d3fk.h: D = x0_hat + c*(x0_hat - x0_prev) stands in for x0_hat in
+// the update above, and x0_prev <- x0_hat for the next step.  With c == 0 x0_prev is only written (D is x0_hat itself),
+// so the result is the posterior kernel's bit for bit and a step needs 16 B/element; with c != 0, 20 B/element.
+static_assert(sizeof(d3fk_posterior_2m_params) == 128 && offsetof(d3fk_posterior_2m_params, x0_prev) == 112 &&
+              offsetof(d3fk_posterior_2m_params, c) == 120 && sizeof(d3fk_op) == 480, "d3fk_posterior_2m_params ABI");
+struct Posterior2mCoefs {
+  PosteriorCoefs b;
+  float c;
+};
+__device__ __forceinline__ Posterior2mCoefs posterior_2m_coefs(const d3fk_posterior_2m_params& p) {
+  const d3fk_posterior_params& q = p.base;
+  Posterior2mCoefs c{{q.k_xi, q.k_x0, q.sigma, q.r_prev, q.offset}, p.c};
+  if (q.coef_table) {
+    const int s = *q.step;
+    const float* row = q.coef_table + 5 * s;
+    c.b.k_xi = row[0];
+    c.b.k_x0 = row[1];
+    c.b.sigma = row[2];
+    c.b.r_prev = row[3];
+    c.c = row[4];
+    c.b.off += (uint64_t)s;
+  }
+  return c;
+}
+// D = fma(c, h - p, h), the difference rounded first.
+__device__ __forceinline__ float4 multistep4(float c, float4 h, float4 p) {
+  return make_float4(__fmaf_rn(c, __fsub_rn(h.x, p.x), h.x), __fmaf_rn(c, __fsub_rn(h.y, p.y), h.y),
+                     __fmaf_rn(c, __fsub_rn(h.z, p.z), h.z), __fmaf_rn(c, __fsub_rn(h.w, p.w), h.w));
+}
+
+__global__ void posterior_2m_kernel(d3fk_posterior_2m_params p) {
+  pdl_enter();
+  const Posterior2mCoefs c = posterior_2m_coefs(p);
+  const d3fk_posterior_params& q = p.base;
+  float4* prev = reinterpret_cast<float4*>(p.x0_prev);
+  const long long nvec = q.n / 4;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < nvec; i += (long long)gridDim.x * blockDim.x) {
+    float4 x = reinterpret_cast<const float4*>(q.x)[i];
+    float4 h = __ldg(reinterpret_cast<const float4*>(q.x0_hat) + i);
+    float4 d = h;
+    if (c.c != 0.f) d = multistep4(c.c, h, prev[i]);
+    prev[i] = h;
+    float4 o = posterior4(c.b.k_xi, x, c.b.k_x0, d);
+    if (c.b.sigma != 0.f) {
+      float4 z;
+      if (q.z) z = __ldg(reinterpret_cast<const float4*>(q.z) + i);
+      else z = philox_normal4(q.seed, (uint64_t)i, c.b.off);
+      posterior_add_noise4(o, c.b.sigma, z);
+    }
+    reinterpret_cast<float4*>(q.x)[i] = o;
+  }
+}
+
+// Masked form: posterior_masked_kernel with D for x0_hat; all-0 mask vectors read no x0_hat and leave x0_prev as it is.
+__global__ void __launch_bounds__(256) posterior_2m_masked_kernel(d3fk_posterior_2m_params p) {
+  pdl_enter();
+  const Posterior2mCoefs cc = posterior_2m_coefs(p);
+  const PosteriorCoefs& c = cc.b;
+  const d3fk_posterior_params& q = p.base;
+  float4* prev = reinterpret_cast<float4*>(p.x0_prev);
+  const float a = sqrtf(1.f - c.r_prev), s = sqrtf(c.r_prev);
+  const int b = blockIdx.y;
+  const unsigned vpp = (unsigned)q.hw / 4u, vps = (unsigned)q.chw / 4u;
+  const long long base = (long long)b * vps;
+  const float4* mask = reinterpret_cast<const float4*>(q.mask) + (long long)b * vpp;
+  for (unsigned v = blockIdx.x * blockDim.x + threadIdx.x; v < vps; v += gridDim.x * blockDim.x) {
+    float4 m = __ldg(mask + v % vpp);
+    m = make_float4(clamp01(m.x), clamp01(m.y), clamp01(m.z), clamp01(m.w));
+    const bool all1 = m.x == 1.f && m.y == 1.f && m.z == 1.f && m.w == 1.f;
+    const bool all0 = m.x == 0.f && m.y == 0.f && m.z == 0.f && m.w == 0.f;
+    const long long i = base + v;
+    float4 post = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (!all0) {
+      float4 x = reinterpret_cast<const float4*>(q.x)[i];
+      float4 h = __ldg(reinterpret_cast<const float4*>(q.x0_hat) + i);
+      float4 d = h;
+      if (cc.c != 0.f) d = multistep4(cc.c, h, prev[i]);
+      prev[i] = h;
+      post = posterior4(c.k_xi, x, c.k_x0, d);
+      if (c.sigma != 0.f) {
+        float4 z;
+        if (q.z) z = __ldg(reinterpret_cast<const float4*>(q.z) + i);
+        else z = philox_normal4(q.seed, (uint64_t)i, c.off);
+        posterior_add_noise4(post, c.sigma, z);
+      }
+    }
+    float4 known = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (!all1) {
+      float4 n = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (c.r_prev != 0.f) {
+        if (q.known_noise) n = __ldg(reinterpret_cast<const float4*>(q.known_noise) + i);
+        else n = philox_normal4(q.seed, (uint64_t)i | (1ull << 63), c.off);
+      }
+      float4 x = __ldg(reinterpret_cast<const float4*>(q.src) + i);
+      known = make_float4(blend1(a, x.x, s, n.x), blend1(a, x.y, s, n.y), blend1(a, x.z, s, n.z), blend1(a, x.w, s, n.w));
+    }
+    reinterpret_cast<float4*>(q.x)[i] = make_float4(composite1(m.x, post.x, known.x), composite1(m.y, post.y, known.y),
+                                                    composite1(m.z, post.z, known.z), composite1(m.w, post.w, known.w));
+  }
+}
+
 __global__ void inc_kernel(int* p) {
   pdl_enter(); *p += 1; }
 
@@ -1389,6 +1490,31 @@ int launch_posterior(const d3fk_posterior_params* p, cudaStream_t s) {
   launch_k(posterior_masked_kernel, dim3(gx, (unsigned)(p->n / p->chw)), dim3(256), 0, s, dim3(1, 1, 1), *p);
   count_launch();
   return check_launch("posterior_step");
+}
+static bool overlaps(const void* a, const void* b, long long bytes) {
+  return a && b && (uintptr_t)a < (uintptr_t)b + bytes && (uintptr_t)b < (uintptr_t)a + bytes;
+}
+int launch_posterior_2m(const d3fk_posterior_2m_params* p, cudaStream_t s) {
+  const d3fk_posterior_params* q = &p->base;
+  D3FK_CHECK_ARG(q->n % 4 == 0, "n must be a multiple of 4");
+  D3FK_CHECK_ARG(q->x && q->x0_hat && p->x0_prev, "the 2M posterior needs x, x0_hat and x0_prev");
+  D3FK_CHECK_ARG(!overlaps(p->x0_prev, q->x0_hat, q->n * 4) && !overlaps(p->x0_prev, q->x, q->n * 4),
+                 "x0_prev must not overlap x0_hat or x");
+  D3FK_CHECK_ARG(((uintptr_t)p->x0_prev & 15) == 0, "x0_prev must be 16-byte aligned");
+  if (!q->mask) {
+    launch_k(posterior_2m_kernel, dim3(grid_for(q->n / 4, 256)), dim3(256), 0, s, dim3(1, 1, 1), *p);
+    count_launch();
+    return check_launch("posterior_2m_step");
+  }
+  D3FK_CHECK_ARG(q->src, "the masked posterior needs src");
+  D3FK_CHECK_ARG(q->hw > 0 && q->hw % 4 == 0 && q->chw >= q->hw && q->chw % q->hw == 0, "hw must be a multiple of 4 dividing chw");
+  D3FK_CHECK_ARG(q->n > 0 && q->n % q->chw == 0 && q->n / q->chw <= 65535, "n must be 1..65535 samples of chw elements");
+  D3FK_CHECK_ARG((((uintptr_t)q->x | (uintptr_t)q->x0_hat | (uintptr_t)q->src | (uintptr_t)q->mask | (uintptr_t)q->z |
+                   (uintptr_t)q->known_noise) & 15) == 0, "buffers must be 16-byte aligned");
+  const int gx = cdiv(q->chw / 4, 256);
+  launch_k(posterior_2m_masked_kernel, dim3(gx, (unsigned)(q->n / q->chw)), dim3(256), 0, s, dim3(1, 1, 1), *p);
+  count_launch();
+  return check_launch("posterior_2m_step");
 }
 int launch_inc(const d3fk_misc_params* p, cudaStream_t s) {
   launch_k(inc_kernel, dim3(1), dim3(1), 0, s, dim3(1, 1, 1), (int*)p->p0);

@@ -58,9 +58,49 @@ def q_sample(batch, lam, noise=None, y=None, seed=0, offset=0, fixed_r=None, ret
     return out
 
 
-def noise_ratio_grid(n_steps, r_start=1.0):
-    """r_N = r_start > ... > r_0 = 0, linear in r (alpha_bar = 1 - r)."""
-    return [r_start * (1.0 - i / n_steps) for i in range(n_steps + 1)]
+def noise_ratio_grid(n_steps, r_start=1.0, kind="linear", r_min=1e-3):
+    """The sampler's ratios r_start = grid[0] > ... > grid[n_steps] = 0.
+    kind="linear": linear in r (alpha_bar = 1 - r).
+    kind="logsnr": uniform in lambda(r) = ln((1 - r)/r)/2 from lambda(min(r_start, 1 - r_min)) to lambda(r_min) over the
+    first n_steps points, then 0; grid[0] is r_start itself, so from r_start = 1 the first step goes straight from pure
+    noise to the second point.  n_steps = 1 is [r_start, 0].  The last nonzero ratio is r_min whatever n_steps, so the
+    trajectory ends at the same point for every step count (the linear grid's ends at r_start/n_steps)."""
+    if kind == "linear":
+        return [r_start * (1.0 - i / n_steps) for i in range(n_steps + 1)]
+    if kind != "logsnr":
+        raise ValueError(f"unknown grid kind {kind!r}: 'linear' or 'logsnr'")
+    if n_steps < 1:
+        raise ValueError(f"n_steps must be at least 1, got {n_steps}")
+    if not 0.0 < r_min < 0.5:
+        raise ValueError(f"r_min must lie in (0, 0.5), got {r_min}")
+    r_start = float(r_start)
+    if not 0.0 <= r_start <= 1.0:
+        raise ValueError(f"r_start must lie in [0, 1], got {r_start}")
+    if r_start == 0.0:
+        return [0.0] * (n_steps + 1)
+    if n_steps == 1:
+        return [r_start, 0.0]
+    if r_start <= r_min:
+        raise ValueError(f"a logsnr grid of {n_steps} steps needs r_start > r_min = {r_min}, got {r_start}")
+    la, lb = log_snr(min(r_start, 1.0 - r_min)), log_snr(r_min)
+    grid = [ratio_of_log_snr(la + (lb - la) * k / (n_steps - 1)) for k in range(n_steps)] + [0.0]
+    grid[0] = r_start
+    return grid
+
+
+def log_snr(r):
+    """lambda(r) = ln((1 - r)/r)/2: -inf at r = 1, +inf at r = 0."""
+    r = float(r)
+    if r >= 1.0:
+        return -math.inf
+    if r <= 0.0:
+        return math.inf
+    return 0.5 * math.log((1.0 - r) / r)
+
+
+def ratio_of_log_snr(lam):
+    """The inverse of log_snr: r = 1/(1 + e^{2 lambda})."""
+    return 1.0 / (1.0 + math.exp(2.0 * lam))
 
 
 def posterior_coeffs(r_i, r_prev, eta):
@@ -90,6 +130,52 @@ def posterior_coef_table(grid, eta):
     return rows
 
 
+def dpmpp_2m_coeffs(r_before, r_i, r_prev, eta):
+    """(k_xi, k_x0, sigma, c) of the second-order multistep (DPM-Solver++ 2M) step from r_i to r_prev = r_t, whose
+    previous step started at r_before (None on the first step):
+        D = x0_hat + c*(x0_hat - x0_hat of the previous step),   x_t = k_xi*x_i + k_x0*D + sigma*z
+        k_xi = (s_t/s_i) e^{-eta h},  k_x0 = alpha_t (1 - e^{-(1+eta) h}),  sigma = s_t sqrt(1 - e^{-2 eta h}),
+        c = h/(2 h_before),  h = lambda(r_t) - lambda(r_i),  h_before = lambda(r_i) - lambda(r_before)
+    with alpha = sqrt(1 - r), s = sqrt(r), lambda = log_snr.  This is k-diffusion's dpmpp_2m at eta = 0 and its
+    dpmpp_2m_sde (midpoint) at eta > 0.  At eta = 0 and eta = 1, (k_xi, k_x0, sigma) equal posterior_coeffs (DDIM and
+    DDPM ancestral); for 0 < eta < 1 it is k-diffusion's family of noise levels, not the DDIM-eta one.  c = 0 (the
+    first-order update) on the first step and where h or h_before is infinite (from r = 1, the step after it, the step to
+    r = 0).  A step to r_t = 0, or from r_i = 0, returns x0_hat: (0, 1, 0, 0)."""
+    r_i, r_t, eta = float(r_i), float(r_prev), float(eta)
+    if r_t <= 0.0 or r_i <= 0.0:
+        return 0.0, 1.0, 0.0, 0.0
+    h = log_snr(r_t) - log_snr(r_i)
+    a_t, s_t = math.sqrt(1.0 - r_t), math.sqrt(r_t)
+    if math.isinf(h):                          # from r_i = 1: s_i = 1 and every e^{-k h} with k > 0 is 0
+        k_xi = s_t if eta == 0.0 else 0.0
+        k_x0 = a_t
+        sigma = s_t if eta > 0.0 else 0.0
+    else:
+        k_xi = s_t / math.sqrt(r_i) * math.exp(-eta * h)
+        k_x0 = -a_t * math.expm1(-(1.0 + eta) * h)
+        sigma = s_t * math.sqrt(-math.expm1(-2.0 * eta * h))
+    c = 0.0
+    if r_before is not None:
+        h_before = log_snr(r_i) - log_snr(r_before)
+        if math.isfinite(h) and math.isfinite(h_before) and h_before != 0.0:
+            c = h / (2.0 * h_before)
+    return k_xi, k_x0, sigma, c
+
+
+def dpmpp_2m_coef_table(grid, eta):
+    """Rows (k_xi, k_x0, sigma, r_prev, c) of the 2M sampler's device coefficient table, one per step i from grid[i] to
+    grid[i + 1]: posterior_coef_table's four columns with dpmpp_2m_coeffs's coefficients, and c.  The last row is
+    (0, 1, 0, 0, 0) (x0_hat), as is every row of a grid of zeros."""
+    rows = []
+    for i in range(len(grid) - 1):
+        if grid[i] <= 0.0:
+            rows.append((0.0, 1.0, 0.0, 0.0, 0.0))
+            continue
+        k_xi, k_x0, sigma, c = dpmpp_2m_coeffs(grid[i - 1] if i > 0 else None, grid[i], grid[i + 1], eta)
+        rows.append((k_xi, k_x0, sigma, max(float(grid[i + 1]), 0.0), c))
+    return rows
+
+
 def normalize_mask(mask, batch, height, width):
     """An inpainting mask as the contiguous float32 [B,1,H,W] buffer the masked posterior reads (1 = generate, 0 = keep,
     fractions feather; the kernel clamps to [0, 1]).  Accepts [H,W], [1,1,H,W] or [B,1,H,W], float32 or bool, on any
@@ -115,6 +201,43 @@ def posterior_step_(x_i, x0_hat, r_i, r_prev, z=None, eta=0.0, seed=0, offset=0,
     if not x_i.is_contiguous() or not x0_hat.is_contiguous():
         raise ValueError("posterior_step_ needs contiguous tensors")
     k_xi, k_x0, sigma = posterior_coeffs(float(r_i), float(r_prev), eta)
+    masked, _keep = _masked_fields(x_i, r_prev, src, mask, known_noise)
+    op = make_op(_lib.OP_POSTERIOR, n=x_i.numel(), x=x_i.data_ptr(), x0_hat=x0_hat.data_ptr(),
+                 z=None if z is None else z.contiguous().data_ptr(), k_xi=k_xi, k_x0=k_x0, sigma=sigma,
+                 seed=int(seed), offset=int(offset), **masked)
+    _lib.run_single(op, _stream(x_i))
+    return x_i
+
+
+def dpmpp_2m_step_(x_i, x0_hat, x0_prev, r_before, r_i, r_prev, z=None, eta=0.0, seed=0, offset=0, src=None, mask=None,
+                   known_noise=None):
+    """In-place second-order multistep (DPM-Solver++ 2M) update of x_i from r_i to r_prev, one fused kernel: x0_hat is
+    extrapolated with the previous step's, x0_prev (r_before: that step's start ratio, None on the first step), with the
+    coefficients of dpmpp_2m_coeffs; then x0_prev <- x0_hat for the next step.  Where c = 0 x0_prev is not read (any
+    contents), and the result is posterior_step_'s with the same coefficients.  z, seed, offset and the masked form
+    (src, mask, known_noise; all-0 mask vectors leave x0_prev as it is) are posterior_step_'s.  x0_hat may be x_i
+    itself; x0_prev must be a buffer of its own."""
+    _require_cuda_f32(x_i, "x_i")
+    if not x_i.is_contiguous() or not x0_hat.is_contiguous():
+        raise ValueError("dpmpp_2m_step_ needs contiguous tensors")
+    if (not torch.is_tensor(x0_prev) or x0_prev.dtype != torch.float32 or x0_prev.shape != x_i.shape
+            or x0_prev.device != x_i.device or not x0_prev.is_contiguous()):
+        raise ValueError(f"x0_prev must be a contiguous float32 tensor of x_i's shape {tuple(x_i.shape)} on {x_i.device}")
+    if x0_prev.data_ptr() in (x0_hat.data_ptr(), x_i.data_ptr()):
+        raise ValueError("x0_prev must not alias x0_hat or x_i")
+    k_xi, k_x0, sigma, c = dpmpp_2m_coeffs(r_before, float(r_i), float(r_prev), eta)
+    masked, _keep = _masked_fields(x_i, r_prev, src, mask, known_noise)
+    op = make_op(_lib.OP_POSTERIOR_2M, x0_prev=x0_prev.data_ptr(), c=c,
+                 base=dict(n=x_i.numel(), x=x_i.data_ptr(), x0_hat=x0_hat.data_ptr(),
+                           z=None if z is None else z.contiguous().data_ptr(), k_xi=k_xi, k_x0=k_x0, sigma=sigma,
+                           seed=int(seed), offset=int(offset), **masked))
+    _lib.run_single(op, _stream(x_i))
+    return x_i
+
+
+def _masked_fields(x_i, r_prev, src, mask, known_noise):
+    """The masked-form fields of d3fk_posterior_params for posterior_step_ / dpmpp_2m_step_ (empty without a mask), and
+    the tensors they point at, which the caller keeps alive until the launch is enqueued."""
     masked = {}
     if mask is None:
         if src is not None or known_noise is not None:
@@ -143,11 +266,7 @@ def posterior_step_(x_i, x0_hat, r_i, r_prev, z=None, eta=0.0, seed=0, offset=0,
         known_noise = None if known_noise is None else known_noise.contiguous()
         masked = dict(r_prev=r_prev_k, src=src.data_ptr(), mask=mask.data_ptr(),
                       known_noise=None if known_noise is None else known_noise.data_ptr(), chw=x_i[0].numel(), hw=H * W)
-    op = make_op(_lib.OP_POSTERIOR, n=x_i.numel(), x=x_i.data_ptr(), x0_hat=x0_hat.data_ptr(),
-                 z=None if z is None else z.contiguous().data_ptr(), k_xi=k_xi, k_x0=k_x0, sigma=sigma,
-                 seed=int(seed), offset=int(offset), **masked)
-    _lib.run_single(op, _stream(x_i))
-    return x_i
+    return masked, (src, mask, known_noise)
 
 
 def adam_scalars(lr, beta1, beta2, step, ema_decay=0.0):

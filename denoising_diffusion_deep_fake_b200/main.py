@@ -218,7 +218,11 @@ def modify(config_path, checkpoint_path, synthetic, size, checkpoint_dir):
               "sets the batch and size)")
 @click.option("--mask", default=None, help="torch.save'd mask [H,W], [1,1,H,W] or [B,1,H,W]: 1 = generate, 0 = keep "
               "the source, fractions feather")
-def sample(checkpoint_path, which, steps, batch, size, eta, r_start, seed, out, source, mask):
+@click.option("--solver", default="posterior", type=click.Choice(["posterior", "dpmpp-2m"]),
+              help="posterior = first-order update; dpmpp-2m = second-order multistep DPM-Solver++ 2M")
+@click.option("--schedule", default=None, type=click.Choice(["linear", "logsnr"]),
+              help="noise-ratio grid (default: linear for posterior, logsnr for dpmpp-2m)")
+def sample(checkpoint_path, which, steps, batch, size, eta, r_start, seed, out, source, mask, solver, schedule):
     """Iterative reverse-diffusion sampling with CUDA-graph replayed steps (new entry point).  With --source and --mask
     the sampler regenerates only the masked region and keeps the source outside it (masked face swap)."""
     from .sampler import Sampler
@@ -236,15 +240,16 @@ def sample(checkpoint_path, which, steps, batch, size, eta, r_start, seed, out, 
     else:
         model = Unet()
     model = model.to(dev).eval()
+    method = dict(solver=solver.replace("-", "_"), schedule=schedule)
     if source is None:
-        smp = Sampler(model, batch, size, size, steps, r_start=r_start, eta=eta, seed=seed)
+        smp = Sampler(model, batch, size, size, steps, r_start=r_start, eta=eta, seed=seed, **method)
         x0 = smp.run()
     else:
         src = torch.load(source, map_location="cpu").to(dev, torch.float32).contiguous()
         if src.dim() != 4 or src.shape[1] != 3:
             raise click.UsageError(f"--source must hold [B,3,H,W] images, got {tuple(src.shape)}")
         B, _, H, W = src.shape
-        smp = Sampler(model, B, H, W, steps, r_start=r_start, eta=eta, seed=seed, masked=True)
+        smp = Sampler(model, B, H, W, steps, r_start=r_start, eta=eta, seed=seed, masked=True, **method)
         x0 = smp.run(src=src, mask=torch.load(mask, map_location="cpu"))
     torch.save(x0.cpu(), out)
     print(f"wrote {tuple(x0.shape)} samples to {out}")

@@ -247,6 +247,25 @@ typedef struct d3fk_posterior_params {
   int32_t chw, hw;
 } d3fk_posterior_params;
 
+/* ---- second-order multistep update (DPM-Solver++ 2M in data-prediction form; k-diffusion's dpmpp_2m at eta = 0 and
+ * dpmpp_2m_sde, midpoint, at eta > 0), in the variance-preserving ratio r: lambda(r) = ln((1 - r)/r)/2 (-inf at r = 1,
+ * +inf at 0), alpha = sqrt(1 - r), s = sqrt(r).  Step i goes from r_i to r_t with h_i = lambda(r_t) - lambda(r_i):
+ *   D_i     = x0_i + c_i*(x0_i - x0_{i-1})                       (x0_{i-1}: the previous step's x0_hat, kept in x0_prev)
+ *   x_{i+1} = k_xi*x_i + k_x0*D_i + sigma*z
+ *   k_xi = (s_t/s_i) e^{-eta h},  k_x0 = alpha_t (1 - e^{-(1+eta) h}),  sigma = s_t sqrt(1 - e^{-2 eta h}),
+ *   c_i  = h_i / (2 h_{i-1})
+ * c_i = 0 on the first step and wherever h_i or h_{i-1} is infinite; a step to r_t = 0 is (0, 1, 0, 0, 0) and returns
+ * x0_hat.  At eta = 0 and eta = 1 (k_xi, k_x0, sigma) equal the first-order posterior's, so a row with c = 0 is today's
+ * update.  Rounding: d = h - p, D = fma(c, d, h), then the posterior's (fma(k_xi, x, k_x0*D), fma(sigma, z, .)): with
+ * c = 0 the result is bit-identical to d3fk_posterior_step with the same coefficients, and x0_prev is not read.
+ * Every vector whose update is computed copies x0_hat into x0_prev (the masked form skips all-0 mask vectors, which
+ * read no x0_hat either).  z and the masked known noise are the posterior's streams.  Table form: base.coef_table rows
+ * are 5 floats (k_xi, k_x0, sigma, r_prev, c) indexed by *base.step.  x0_hat may alias x, never x0_prev. */
+typedef struct d3fk_posterior_2m_params {
+  d3fk_posterior_params base;
+  float* x0_prev; float c; int32_t _pad;
+} d3fk_posterior_2m_params;   /* 128 bytes */
+
 typedef struct d3fk_misc_params {          /* MEMSET: p0[0..n) bytes = 0; INC: *(int32*)p0 += 1; PACK_ALL: see enum */
   void* p0; int64_t n;
 } d3fk_misc_params;
@@ -304,8 +323,9 @@ enum d3fk_op_kind {
                             frozen: ONE streaming pass writes dx (and dres) and accumulates bstats, then bn_bwd_finalize writes dgamma / dbeta */
   D3FK_OP_NCHW2S2D = 31,   /* layout params (C = 3, cpad = 4, H and W even): fp32 NCHW -> the padded space-to-depth image of conv mode 2:
                               dst[b][h/2][w/2 + 2][((h%2)*2 + (w%2))*4 + c]; the pad pixels / channel are left untouched (zero them once) */
-  D3FK_OP_PACK_STEM = 32   /* pack params (Cout, Cin = 3, kh = kw = 7): w_fwd[co][th*64 + tw*16 + (dy*2+dx)*4 + ci] =
+  D3FK_OP_PACK_STEM = 32,  /* pack params (Cout, Cin = 3, kh = kw = 7): w_fwd[co][th*64 + tw*16 + (dy*2+dx)*4 + ci] =
                               w[co][ci][2*th+dy-1][2*tw+dx-1] (0 outside the 7x7 window and for ci = 3): the conv mode 2 weights */
+  D3FK_OP_POSTERIOR_2M = 33   /* posterior_2m params: the second-order multistep update (5-float table rows) */
 };
 
 /* `lane`: 0 = the caller's stream (the main chain).  lane 1..D3FK_MAX_LANES = an internal branch stream: the op runs there,
@@ -323,7 +343,7 @@ typedef struct d3fk_op {
     d3fk_qsample_params qsample; d3fk_posterior_params posterior; d3fk_misc_params misc;
     d3fk_adam_params adam; d3fk_loss_params loss; d3fk_convbn_params convbn; d3fk_upcat_params upcat;
     d3fk_wgrad_group_params wgrad_group; d3fk_frames_params frames; d3fk_affine_qsample_params affine_qsample;
-    d3fk_scalars_params scalars;
+    d3fk_scalars_params scalars; d3fk_posterior_2m_params posterior_2m;
   } u;
 } d3fk_op;
 
@@ -373,6 +393,7 @@ int d3fk_chansum(const d3fk_chansum_params* p, d3fk_stream stream);
 int d3fk_upcat(const d3fk_upcat_params* p, d3fk_stream stream);
 int d3fk_q_sample(const d3fk_qsample_params* p, d3fk_stream stream);
 int d3fk_posterior_step(const d3fk_posterior_params* p, d3fk_stream stream);
+int d3fk_posterior_2m_step(const d3fk_posterior_2m_params* p, d3fk_stream stream);
 int d3fk_adam(const d3fk_adam_params* p, d3fk_stream stream);
 int d3fk_set_scalars(const d3fk_scalars_params* p, d3fk_stream stream);
 int d3fk_mse_ssim_loss(const d3fk_loss_params* p, d3fk_stream stream);
